@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py — BN254 G1 MSM throughput (Mpoints/s) on B200 and Groth16 prove latency, the metric BASELINE.json names.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--quick]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--quick] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
+
+The run writes nothing into the source tree (it may be read-only): no bytecode, and the CPU oracle's -march=native build goes to a temp dir.
+--dump-outputs DIR writes what the timed path computed in its last step, as affine points: the headline MSM's result (DIR/msm_affine.npy) or,
+with --workload groth16, the proof (DIR/proof_{a,b,c}.npy), so that two builds can be compared output for output on the same seeded inputs.
 
 Inputs (both arms, every N): bases P_i = k_i * G with k_i = from_u512(splitmix64 stream of (BASE_SEED, i)) — generated on the device by
 kgr_bases_generate_at in our arm and by the oracle's restatement of the same stream in the reference arm — and scalars s_i drawn by numpy
@@ -457,7 +461,7 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
-def groth16_record(args):
+def groth16_record(args, steps=5, warmup=5, cpu_steps=1, cpu_warmup=0):
     import contextlib
     import importlib.util
     import io
@@ -469,32 +473,42 @@ def groth16_record(args):
         # Measured twice.  In a process that has not run any multi-threaded CPU work yet the call is ~25 % slower however many warm-up proofs
         # precede it (the per-lane host threads run on cores at idle clocks; tools/probe_prover_host.py).  The second pass runs after the CPU
         # baseline of the first has used all host cores, which is the state of a prover process that has generated a witness; both figures are reported.
-        rows.bench_groth16(args.logm, out)
-        rows.bench_groth16(args.logm, out)
-    return out[1], out[0]
+        rows.bench_groth16(args.logm, out, steps, warmup, cpu_steps, cpu_warmup)
+        proof = rows.bench_groth16(args.logm, out, steps, warmup, cpu_steps, cpu_warmup)
+    return out[1], out[0], proof
 
 
 def run_groth16(args, rank):
     """Groth16 prove latency (BASELINE metric, second half; config #4 scaled as SURVEY H7 suggests): create_proof after witness generation —
     7 FFTs, six G1 and two G2 MSMs, assembly of A, B, C — on the chained x^3 + x + 5 circuit with 2^logm constraints, host buffers in, three
     affine points out.  `--impl reference` times the restated reference code on the same inputs (FFT halves forked like rayon::join, the eight MSMs on all
-    cores).  The proof is checked against its discrete logs computed from the toxic waste."""
+    cores).  Either arm takes the best of --steps timed runs after --warmup warm-up runs.  The proof is checked against its discrete logs
+    computed from the toxic waste; --dump-outputs writes it (ours only)."""
     if rank != 0:
         return
     import kogarashi_b200 as k
     k.init([int(os.environ.get("LOCAL_RANK", "0"))])
-    rec, first = groth16_record(args)
-    cpu_ms = rec["cpu_baseline"]["total_seconds"] * 1e3
     ours = args.impl != "reference"
+    if ours:
+        rec, first, proof = groth16_record(args, steps=args.steps, warmup=args.warmup)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"proof_a": proof[0], "proof_b": proof[1], "proof_c": proof[2]})
+        timing = f"wall clock around Groth16Prover.prove_from_evaluations, best of {args.steps} after {args.warmup} warm-up proofs; CRS registered on the GPU"
+        cpu_sample = "the whole workload once: "
+    else:
+        rec, first, _ = groth16_record(args, cpu_steps=args.steps, cpu_warmup=args.warmup)
+        timing = f"wall clock around the restated reference H pipeline and the eight MSMs, best of {args.steps} after {args.warmup} warm-up runs"
+        cpu_sample = f"the whole workload, best of {args.steps} after {args.warmup} warm-up runs: "
+    cpu_ms = rec["cpu_baseline"]["total_seconds"] * 1e3
     value = rec["gpu_wall_ms"]["normal"] if ours else cpu_ms
-    line = {"metric": "groth16_prove_latency", "value": value, "unit": "ms", "n_gpus": 1, "steps": 5, "warmup": 5, "ms_per_step": value, "higher_is_better": False,
+    line = {"metric": "groth16_prove_latency", "value": value, "unit": "ms", "n_gpus": 1, "steps": args.steps, "warmup": args.warmup, "ms_per_step": value, "higher_is_better": False,
             "scaling": "weak", "vs_baseline": None, "dtype": "u32 limbs (Montgomery Fq/Fr/Fq2)" if ours else "u64 limbs (Montgomery)", "data": "synthetic",
             "config": workload_config(args, 1),
-            "timing": "wall clock around Groth16Prover.prove_from_evaluations, best of 5 after 5 warm-up proofs; CRS registered on the GPU",
+            "timing": timing,
             "e2e": {"value": value, "unit": "ms", "h2d_bytes_per_step": (3 * rec["constraints"] + 4 * rec["constraints"]) * 32 if ours else 0,
                     "d2h_bytes_per_step": (1 << rec["log_n"]) * 32 if ours else 0},
             "cpu_baseline": {"value": cpu_ms, "unit": "ms", "cores": rec["cpu_baseline"]["cores"], "kind": "port",
-                             "sample": "the whole workload once: " + rec["cpu_baseline"]["note"]},
+                             "sample": cpu_sample + rec["cpu_baseline"]["note"]},
             "roofline": None, "proof_checked_against_discrete_logs": rec["checked_against_discrete_logs"], "h_bit_exact_with_oracle": rec["h_bit_exact_with_oracle"]}
     if ours:
         line["gpu_launches"] = int(k.launch_count(0))
@@ -512,7 +526,19 @@ def strip(rec):
     return rec
 
 
+def dump_outputs(dirname, points):
+    """points: {name: affine point (x, y as Montgomery limbs, then is_infinity)} -> DIR/<name>.npy, each a float64 array of shape (words, 2)
+    holding every uint64 limb as its low and high 32-bit halves, which float64 holds exactly.  Points are stored in affine form, not as the
+    projective X, Y, Z the MSM engine returns: the sort places a bucket's points with atomic cursors, so their order and with it the
+    projective representative of the same group element change from run to run; the affine form depends on the inputs alone."""
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in points.items():
+        a = np.asarray(a, dtype=np.uint64)
+        np.save(os.path.join(dirname, name + ".npy"), np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1).astype(np.float64))
+
+
 def main():
+    sys.dont_write_bytecode = True  # the modules this run imports leave no __pycache__ in the tree
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=10)
@@ -527,7 +553,17 @@ def main():
     ap.add_argument("--workload", default="msm", choices=["msm", "groth16"],
                     help="groth16 = the other half of BASELINE's metric: prove latency (create_proof after witness generation) on the chained example circuit")
     ap.add_argument("--logm", type=int, default=16, help="log2 of the constraint count for --workload groth16")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path computed in its last step: the MSM result as DIR/msm_affine.npy, or with --workload groth16 the "
+                         "proof as DIR/proof_{a,b,c}.npy. Points are stored in affine form (x, y, is_infinity), not as the projective X, Y, Z the "
+                         "engine returns, whose representative changes from run to run with the order of the bucket additions; float64, each uint64 "
+                         "limb as its low and high 32-bit halves")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours: the reference arm's sample size is chosen by a timing calibration, so its result "
+                 "is not a fixed function of the arguments")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -568,8 +604,10 @@ def main():
 
     if world == 1:
         sampler = ClockSampler(local_rank)
-        rec, ms_per_step, _ = measure_single(k, torch, args.curve, args.logn, args.steps, args.warmup, local_rank, flush, want_e2e=True, full_cpu=args.logn <= 20,
-                                             cpu_sample_logn=args.cpu_sample_logn, sampler=sampler, want_precompute=not args.quick)
+        rec, ms_per_step, aff = measure_single(k, torch, args.curve, args.logn, args.steps, args.warmup, local_rank, flush, want_e2e=True, full_cpu=args.logn <= 20,
+                                               cpu_sample_logn=args.cpu_sample_logn, sampler=sampler, want_precompute=not args.quick)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"msm_affine": aff})
         clocks = rec["clocks"]
         line = dict(common)
         line.update({"value": rec["value"], "ms_per_step": ms_per_step, "scaling": "weak", "l2": "flushed between steps (512 MiB write)",
@@ -618,7 +656,7 @@ def main():
             except Exception as ex:
                 line["ntt_2p20"] = {"error": repr(ex)}
             try:
-                g16, first = groth16_record(args)
+                g16, first, _ = groth16_record(args)
                 line["groth16_2p16"] = {"metric": "groth16_prove_latency", "unit": "ms", "value": g16["gpu_wall_ms"]["normal"], "idle_host_ms": first["gpu_wall_ms"]["normal"],
                                         "precomputed_crs_tables_ms": g16["gpu_wall_ms"]["precomputed"], "constraints": g16["constraints"],
                                         "cpu_baseline": {"value": g16["cpu_baseline"]["total_seconds"] * 1e3, "unit": "ms", "cores": g16["cpu_baseline"]["cores"], "kind": "port",
@@ -631,7 +669,7 @@ def main():
             try:  # SURVEY 8(f) row N4: one Nova IVC step's vector work on one curve (commit(W), cross term, commit(T), two folds), state resident on the GPU
                 import subprocess
                 env = dict(os.environ, CUDA_VISIBLE_DEVICES=os.environ.get("CUDA_VISIBLE_DEVICES", str(local_rank)))
-                outp = subprocess.run([sys.executable, os.path.join(ROOT, "tools", "bench_ivc_step.py"), "15", "1"], capture_output=True, text=True, timeout=300, env=env)
+                outp = subprocess.run([sys.executable, "-B", os.path.join(ROOT, "tools", "bench_ivc_step.py"), "15", "1"], capture_output=True, text=True, timeout=300, env=env)
                 recs = [json.loads(l) for l in outp.stdout.splitlines() if l.startswith("{")]
                 line["nova_ivc_step_32k"] = recs[-1] if recs else {"error": (outp.stderr or "no output")[-300:]}
             except Exception as ex:
@@ -646,6 +684,8 @@ def main():
 
     # ---- N > 1: strong scaling of one MSM -----------------------------------------------------------------------------------------------
     main_rec = measure_strong(k, torch, dist, sharding, args.curve, args.strong_logn, world, rank, args.steps, args.warmup, barrier, sampler=ClockSampler(local_rank))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"msm_affine": main_rec["affine"]})
     extra = {}
     if not args.quick:
         extra["strong_2p24"] = measure_strong(k, torch, dist, sharding, args.curve, 24, world, rank, args.steps, args.warmup, barrier)

@@ -36,24 +36,45 @@ def build(force=False):
     return _LIB_PATH
 
 
+def _owned_private(path, kind):
+    """True if `path` is a `kind` (stat.S_ISDIR / S_ISREG), not a symlink, owned by this user and writable by nobody else: only then is
+    a shared object found there ours to load."""
+    import stat
+    st = os.lstat(path)
+    return kind(st.st_mode) and st.st_uid == os.getuid() and not st.st_mode & (stat.S_IWGRP | stat.S_IWOTH)
+
+
 def _native_path():
-    """libzkstd_oracle.<cpu>.so: the same source built with -march=native on THIS host (the portable .so travels between machines with
-    different CPUs).  Built at first use; None if that is not possible (no compiler), in which case the portable build is used."""
+    """libzkstd_oracle.<tag>.so: the same source built with -march=native on THIS host (the portable .so travels between machines with
+    different CPUs).  Built at first use into the user's cache directory ($XDG_CACHE_HOME or ~/.cache, kogarashi-oracle/), not into the
+    source tree, which a benchmark run must leave as it found it (and which may be read-only); the tag hashes the CPU and the sources, so
+    checkouts of different versions never share a build.  Nothing is loaded from that directory unless it and the file belong to this
+    user and are writable by no one else.  None if any of this is not possible (no compiler, no private cache directory), in which case
+    the portable build is used."""
     if os.environ.get("ZKO_PORTABLE"):
         return None
     try:
         import hashlib
+        import stat
         with open("/proc/cpuinfo") as f:
             model = next((line for line in f if line.startswith(("model name", "flags"))), "")
             flags = next((line for line in f if line.startswith("flags")), "")
-        tag = hashlib.sha1((model + flags).encode()).hexdigest()[:10]
-        path = os.path.join(_HERE, f"libzkstd_oracle.{tag}.so")
-        src = [os.path.join(_HERE, f) for f in ("zkstd_oracle.cpp", "zkstd_oracle.hpp")]
-        if not os.path.exists(path) or any(os.path.getmtime(s) > os.path.getmtime(path) for s in src):
+        h = hashlib.sha1((model + flags).encode())
+        for name in ("zkstd_oracle.cpp", "zkstd_oracle.hpp"):
+            with open(os.path.join(_HERE, name), "rb") as f:
+                h.update(f.read())
+        base = os.environ.get("XDG_CACHE_HOME") or os.path.join(os.path.expanduser("~"), ".cache")
+        cache = os.path.join(base, "kogarashi-oracle")
+        os.makedirs(cache, mode=0o700, exist_ok=True)
+        if not _owned_private(cache, stat.S_ISDIR):
+            return None
+        path = os.path.join(cache, f"libzkstd_oracle.{h.hexdigest()[:10]}.so")
+        if not os.path.lexists(path):
             tmp = f"{path}.{os.getpid()}.tmp"
             subprocess.check_call(["make", "-C", _HERE, "-s", "native", f"OUT={tmp}"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+            os.chmod(tmp, 0o700)
             os.replace(tmp, path)
-        return path
+        return path if _owned_private(path, stat.S_ISREG) else None
     except Exception:
         return None
 

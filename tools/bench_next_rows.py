@@ -57,10 +57,11 @@ def _wall(fn):
     return time.perf_counter() - t0
 
 
-def bench_groth16(logm, out):
-    steps = ((1 << logm) - 1) // 3
+def bench_groth16(logm, out, steps=5, warmup=5, cpu_steps=1, cpu_warmup=0):
+    """GPU: best of `steps` proofs after `warmup` warm-up proofs; CPU baseline: best of `cpu_steps` runs after `cpu_warmup`.  Returns the
+    last proof (A, B, C as affine limb arrays) of the default (not precomputed) prover."""
     t0 = time.perf_counter()
-    cs, _ = G.chain_circuit(steps, 3)
+    cs, _ = G.chain_circuit(((1 << logm) - 1) // 3, 3)
     E, trap, uvw = G.crs_exponents(cs, B.XorShift128(A.DEFAULT_SEED))
     setup_s = time.perf_counter() - t0
     mont = lambda vals: np.array([B.int_to_limbs(B.to_mont(v, B.FR)) for v in vals], dtype=np.uint64).reshape(-1, 4)
@@ -79,14 +80,16 @@ def bench_groth16(logm, out):
     xs, ws = mont(cs.x), mont(cs.w)
     rng = B.XorShift128(bytes(range(1, 17)))
     r, s = rng.random_field(B.FR), rng.random_field(B.FR)
-    res = {}
+    res, proof = {}, None
     for pre in (False, True):
         prover = Groth16Prover(vk[0], vk[1], vk[2], *crs[0], *crs[1], *crs[2], *crs[3], vk2[0], vk2[1], *crs_g2, precompute=pre)
-        for _ in range(5):   # warm-up: lanes, NTT tables, workspaces
+        for _ in range(warmup):   # warm-up: lanes, NTT tables, workspaces
             prover.prove_from_evaluations(E["k"], a_ev, b_ev, c_ev, xs, ws, r, s)
-        wall = min(_wall(lambda: prover.prove_from_evaluations(E["k"], a_ev, b_ev, c_ev, xs, ws, r, s)) for _ in range(5))
+        wall = min(_wall(lambda: prover.prove_from_evaluations(E["k"], a_ev, b_ev, c_ev, xs, ws, r, s)) for _ in range(steps))
         Ap, Bp, Cp, q = prover.prove_from_evaluations(E["k"], a_ev, b_ev, c_ev, xs, ws, r, s)
         res["precomputed" if pre else "normal"] = wall * 1e3
+        if not pre:
+            proof = (Ap, Bp, Cp)
         prover.free()
     q_int = [B.from_mont(B.limbs_to_int(x), B.FR) for x in q]
     a_exp, b_exp, c_exp, pairing_ok = G.expected_exponents(trap, uvw, cs.x, cs.w, q_int, E["n"], r, s)
@@ -96,15 +99,20 @@ def bench_groth16(logm, out):
     # CPU baseline: the same work with the restated reference code (7 FFTs + the six G1 and two G2 MSMs of prover.rs:51-65)
     cores = os.cpu_count() or 1
     l = cs.l
-    t0 = time.perf_counter()
-    q_ref, n_ref = A.groth16_h(E["k"], a_ev, b_ev, c_ev)
-    fft_s = time.perf_counter() - t0
-    t0 = time.perf_counter()
-    for pts_inf, sc in ((crs[2], q_ref[:n_ref]), (crs[3], ws), (crs[0], xs), ((crs[0][0][l:], crs[0][1][l:]), ws), (crs[1], xs), ((crs[1][0][l:], crs[1][1][l:]), ws)):
-        A.msm(A.BN254_G1, pts_inf[0], sc, inf=pts_inf[1], threads=cores)
-    for pts_inf, sc in ((crs_g2, xs), ((crs_g2[0][l:], crs_g2[1][l:]), ws)):
-        A.msm(A.BN254_G2, pts_inf[0], sc, inf=pts_inf[1], threads=cores)
-    msm_s = time.perf_counter() - t0
+    best = None
+    for it in range(cpu_warmup + cpu_steps):
+        t0 = time.perf_counter()
+        q_ref, n_ref = A.groth16_h(E["k"], a_ev, b_ev, c_ev)
+        fft_s = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        for pts_inf, sc in ((crs[2], q_ref[:n_ref]), (crs[3], ws), (crs[0], xs), ((crs[0][0][l:], crs[0][1][l:]), ws), (crs[1], xs), ((crs[1][0][l:], crs[1][1][l:]), ws)):
+            A.msm(A.BN254_G1, pts_inf[0], sc, inf=pts_inf[1], threads=cores)
+        for pts_inf, sc in ((crs_g2, xs), ((crs_g2[0][l:], crs_g2[1][l:]), ws)):
+            A.msm(A.BN254_G2, pts_inf[0], sc, inf=pts_inf[1], threads=cores)
+        msm_s = time.perf_counter() - t0
+        if it >= cpu_warmup and (best is None or fft_s + msm_s < best[0] + best[1]):
+            best = (fft_s, msm_s)
+    fft_s, msm_s = best
     rec = {"row": "N1+N3 Groth16 create_proof after witness generation (7 FFTs + six G1 MSMs + two G2 MSMs + assembly of A, B, C)",
            "constraints": cs.m, "log_n": E["k"], "gpu_wall_ms": res, "checked_against_discrete_logs": bool(ok),
            "h_bit_exact_with_oracle": bool(q.shape[0] == n_ref and (q == q_ref[:n_ref]).all()),
@@ -113,6 +121,7 @@ def bench_groth16(logm, out):
            "speedup_vs_cpu_baseline": {m: (fft_s + msm_s) * 1e3 / v for m, v in res.items()}, "setup_python_s": setup_s}
     out.append(rec)
     print(json.dumps(rec), flush=True)
+    return proof
 
 
 def bench_g2(logn, out):
