@@ -187,6 +187,18 @@ int kgr_host_free(void *p);
 int kgr_groth16_msms(unsigned log_n, const uint64_t *a, const uint64_t *b, const uint64_t *c, size_t m, kgr_bases_t *h, uint64_t *h_out, uint64_t *q_out,
                      size_t *q_len, const kgr_msm_job_t *jobs, size_t n_jobs);
 
+/* groth16/src/prover.rs:32-65 from the constraint system: cs.evaluate() (r1cs.rs:137-142) on the device from the registered shape cs (field 1 = Fr)
+ * and the resident assignment z = cs.x() ++ cs.w() (z->n == n_z of the shape; the first n_inputs elements are the instance, the constant one first),
+ * H as kgr_groth16_h, then the queries with scalars read from z on the device:
+ *   h: q (2^log_n coefficients, never leaving the device)   l: z[n_inputs ..]   a, b_g1, b_g2: z (inputs and aux fused, as prover.rs:58-65)
+ * out: h[12] l[12] a[12] b_g1[12] b_g2[24] projective results (b_g2 == NULL: a G1-only prover, the last 24 words are not written).
+ * jobs: further MSMs with host scalars (the blinding sums) on the other lanes, as in kgr_groth16_msms.  q_out / q_len as there.
+ * Pairs are zipped (msm.rs:25): h min(2^log_n, len), a / b_g1 / b_g2 min(len, n_z), l min(len, n_z - n_inputs); no pairs gives the identity.
+ * Requires 2^log_n >= m (nothing is truncated) and a single-device context: every handle on the first device, unsplit.  Work enqueued on the
+ * library's stream before the call (kgr_vec_fold_device, kgr_nova_cross_term_device writing z) is complete before z is read. */
+int kgr_groth16_prove_r1cs(unsigned log_n, const kgr_r1cs_t *cs, const kgr_vec_t *z, size_t n_inputs, kgr_bases_t *h, kgr_bases_t *l, kgr_bases_t *a,
+                           kgr_bases_t *b_g1, kgr_bases_t *b_g2, uint64_t *out, uint64_t *q_out, size_t *q_len, const kgr_msm_job_t *jobs, size_t n_jobs);
+
 /* Tuning knobs: "window_bits" (0 = auto), "chunk" (entries per accumulate thread, 0 = auto),
  * "reduce_fanin" (power of two), "running_sum_stop" (elements per window below which the reduce
  * switches from running sums to the parallel weighting pass), "final_on_device" (1: Horner over

@@ -148,9 +148,13 @@ void LaunchNtt::h_pointwise(cudaStream_t st, void *a, const void *b, const void 
 // In-place transform with the given twiddle table (forward or inverse): bit reversal + passes.  Returns kernels launched.
 int LaunchNtt::transform(cudaStream_t st, void *d, const void *tw, uint32_t k) {
     if (k == 0) return 0;
+    k_ntt_bitrev<<<cdivu((size_t)1 << k, 256), 256, 0, st>>>((Fr *)d, k);
+    return 1 + transform_bitrev_input(st, d, tw, k);
+}
+int LaunchNtt::transform_bitrev_input(cudaStream_t st, void *d, const void *tw, uint32_t k) {
+    if (k == 0) return 0;
     const uint32_t n = 1u << k;
-    k_ntt_bitrev<<<cdivu(n, 256), 256, 0, st>>>((Fr *)d, k);
-    int launches = 1;
+    int launches = 0;
     const uint32_t np = (k + 9) / 10;
     uint32_t done = 0;
     for (uint32_t p = 0; p < np; p++) {

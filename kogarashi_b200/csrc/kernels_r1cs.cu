@@ -17,7 +17,16 @@ template <class P> __global__ void __launch_bounds__(256) k_vec_fold(uint32_t n,
     body_vec_fold<P>(blockIdx.x * blockDim.x + threadIdx.x, n, a, b, r, out);
 }
 
+__global__ void __launch_bounds__(128) k_r1cs_evaluate(uint32_t k, uint32_t m, Csr a, Csr b, Csr c, const uint32_t *z, uint32_t *out_a, uint32_t *out_b,
+                                                        uint32_t *out_c) {
+    body_r1cs_evaluate<FrP>(blockIdx.x * blockDim.x + threadIdx.x, k, m, a, b, c, z, out_a, out_b, out_c);
+}
+
 static inline unsigned blocks_for(size_t n, unsigned tpb) { return (unsigned)((n + tpb - 1) / tpb); }
+
+void LaunchR1cs::evaluate(cudaStream_t st, uint32_t k, uint32_t m, const Csr &a, const Csr &b, const Csr &c, const uint32_t *z, uint32_t *const out[3]) {
+    k_r1cs_evaluate<<<blocks_for((size_t)1 << k, 128), 128, 0, st>>>(k, m, a, b, c, z, out[0], out[1], out[2]);
+}
 
 void LaunchR1cs::spmv(cudaStream_t st, int field, uint32_t m, const Csr &mat, const uint32_t *z, uint32_t *out) {
     if (!m) return;

@@ -96,6 +96,8 @@ struct LaunchNtt {
     static void scale(cudaStream_t st, void *d, const void *table, const void *c32, uint32_t n);
     static void h_pointwise(cudaStream_t st, void *a, const void *b, const void *c, const void *zinv32, uint32_t n);
     static int transform(cudaStream_t st, void *d, const void *tw, uint32_t k);
+    // the same transform of input already in bit-reversed order: the butterfly passes only
+    static int transform_bitrev_input(cudaStream_t st, void *d, const void *tw, uint32_t k);
 };
 
 // Nova folding vector work (kernels_r1cs.cu).  field: 0 Fq, 1 Fr.
@@ -104,6 +106,8 @@ struct LaunchR1cs {
     static void spmv(cudaStream_t st, int field, uint32_t m, const Csr &mat, const uint32_t *z, uint32_t *out);
     static void cross_term(cudaStream_t st, int field, uint32_t m, const Csr &a, const Csr &b, const Csr &c, const uint32_t *z1, const uint32_t *z2, uint32_t *t);
     static void vec_fold(cudaStream_t st, int field, uint32_t n, const uint32_t *a, const uint32_t *b, const uint32_t r8[8], uint32_t *out);
+    // Groth16 (Fr only): A z, B z, C z over 2^k positions, zero padded, each stored at its bit-reversed index of out[0..2] (2^k elements each)
+    static void evaluate(cudaStream_t st, uint32_t k, uint32_t m, const Csr &a, const Csr &b, const Csr &c, const uint32_t *z, uint32_t *const out[3]);
 };
 
 }  // namespace kgr

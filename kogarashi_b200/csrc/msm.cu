@@ -158,6 +158,7 @@ struct Engine {
     cudaEvent_t ev_pts = nullptr;     // bases of the current oneshot call are on the device
     cudaEvent_t ev_sc = nullptr;      // scalars of the current call are on the device (orders the two uploads)
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;  // fold reduce: the big upper-half sums run on st_copy beside the deep fold levels
+    cudaEvent_t ev_input = nullptr;   // kgr_groth16_prove_r1cs: everything enqueued on st before the call (the resident z) is complete
     bool wait_pts = false;
     cudaEvent_t ev[EV_N] = {};
     cudaEvent_t ev_piece_sc[16] = {}, ev_piece_pts[16] = {};  // piece k's scalars / points are on the device (recorded on st_copy)
@@ -206,6 +207,7 @@ struct Engine {
         CK(cudaEventCreateWithFlags(&ev_sc, cudaEventDisableTiming));
         CK(cudaEventCreateWithFlags(&ev_fork, cudaEventDisableTiming));
         CK(cudaEventCreateWithFlags(&ev_join, cudaEventDisableTiming));
+        CK(cudaEventCreateWithFlags(&ev_input, cudaEventDisableTiming));
         for (auto &e : ev) CK(cudaEventCreate(&e));
         for (auto &e : user_ev) CK(cudaEventCreate(&e));
         for (auto &e : aux_ev) CK(cudaEventCreate(&e));
@@ -250,6 +252,7 @@ struct Engine {
         if (ev_sc) cudaEventDestroy(ev_sc);
         if (ev_fork) cudaEventDestroy(ev_fork);
         if (ev_join) cudaEventDestroy(ev_join);
+        if (ev_input) cudaEventDestroy(ev_input);
         dev = -1;
     }
 };
@@ -812,6 +815,7 @@ struct kgr_bases {
 struct kgr_r1cs {
     int field = 0;
     size_t m = 0, n_z = 0;
+    uint64_t generation = 0;  // kgr_init that created it (checked by kgr_groth16_prove_r1cs)
     kgr::DevBuf<uint32_t> row_ptr[3], cols[3], coeffs[3], z1, z2, t;
     float ms[3] = {0, 0, 0};  // last cross term: H2D of z1 / z2, kernel, commit MSM
     kgr::Csr csr(int i) const { return kgr::Csr{row_ptr[i].p, cols[i].p, coeffs[i].p}; }
@@ -1072,17 +1076,28 @@ static void run_msm(std::vector<Shard> &shards, size_t off, const uint64_t *scal
 }
 
 // ---- kgr_msm_batch: one single-shard MSM per lane, started without waiting and finished later --------------------------
+template <class C> static void lane_enqueue(Engine &e, const Shard &s, size_t off, const uint32_t *d_scalars, int fmt, size_t n) {
+    size_t first = off - s.first;
+    if (s.d_table)
+        enqueue_msm<C>(e, (const AffinePt<C> *)s.d_table, d_scalars, fmt == KGR_SCALARS_MONTGOMERY, (uint32_t)n, s.table_c, (uint32_t)s.count, (uint32_t)first);
+    else
+        enqueue_msm<C>(e, (const AffinePt<C> *)s.d_pts + first, d_scalars, fmt == KGR_SCALARS_MONTGOMERY, (uint32_t)n);
+}
 template <class C> static void lane_start(Engine &e, const Params &P, const Shard &s, size_t off, const uint64_t *scalars, int fmt, size_t n) {
     e.params = P;
     CK(cudaSetDevice(e.dev));
     CK(cudaEventRecord(e.ev[EV_START], e.st));
     e.scalars.ensure(std::max<size_t>(n, 1) * 8);
     upload_from_host(e, e.scalars.p, scalars, n * 32, e.st);
-    size_t first = off - s.first;
-    if (s.d_table)
-        enqueue_msm<C>(e, (const AffinePt<C> *)s.d_table, e.scalars.p, fmt == KGR_SCALARS_MONTGOMERY, (uint32_t)n, s.table_c, (uint32_t)s.count, (uint32_t)first);
-    else
-        enqueue_msm<C>(e, (const AffinePt<C> *)s.d_pts + first, e.scalars.p, fmt == KGR_SCALARS_MONTGOMERY, (uint32_t)n);
+    lane_enqueue<C>(e, s, off, e.scalars.p, fmt, n);
+}
+// Montgomery scalars already on the lane's device; the lane's stream first waits for `ready` (recorded where the scalars were produced)
+template <class C> static void lane_start_device(Engine &e, const Params &P, const Shard &s, size_t off, const uint32_t *d_scalars, size_t n, cudaEvent_t ready) {
+    e.params = P;
+    CK(cudaSetDevice(e.dev));
+    CK(cudaStreamWaitEvent(e.st, ready, 0));
+    CK(cudaEventRecord(e.ev[EV_START], e.st));
+    lane_enqueue<C>(e, s, off, d_scalars, KGR_SCALARS_MONTGOMERY, n);
 }
 template <class C> static void lane_finish(Engine &e, uint64_t *out) {
     CK(cudaSetDevice(e.dev));
@@ -1323,7 +1338,22 @@ static void upload_padded(Engine &e, void *dbuf, const uint64_t *src, size_t n_i
     if (m < n) CK(cudaMemsetAsync((uint8_t *)dbuf + m * 32, 0, (n - m) * 32, e.st));
 }
 
-// prover.rs:36-47 enqueued on e.st: uploads a, b, c (m evaluations each, zero padded), leaves the 2^k coefficients of H in e.ntt_buf[0] (device).
+// prover.rs:36-47 on the three evaluation vectors in e.ntt_buf[0..2] (2^k elements each; in bit-reversed order when bitrev_input), enqueued on
+// e.st: leaves the 2^k coefficients of H in e.ntt_buf[0] (device).
+static void enqueue_groth16_h_transforms(Engine &e, NttDomain &d, bool bitrev_input) {
+    const size_t n = (size_t)1 << d.k;
+    for (int i = 0; i < 3; i++) {
+        // idft then coset_dft (prover.rs:36-41); the 1/n and coset scalings are one elementwise pass
+        if (bitrev_input) e.launches += LaunchNtt::transform_bitrev_input(e.st, e.ntt_buf[i].p, d.inv_tw.p, d.k);
+        else e.launches += LaunchNtt::transform(e.st, e.ntt_buf[i].p, d.inv_tw.p, d.k);
+        LaunchNtt::scale(e.st, e.ntt_buf[i].p, d.cosets.p, &d.n_inv, (uint32_t)n);
+        e.launches += 1 + LaunchNtt::transform(e.st, e.ntt_buf[i].p, d.tw.p, d.k);
+    }
+    LaunchNtt::h_pointwise(e.st, e.ntt_buf[0].p, e.ntt_buf[1].p, e.ntt_buf[2].p, &d.z_inv, (uint32_t)n);  // prover.rs:43-46
+    e.launches++;
+    ntt_enqueue(e, d, e.ntt_buf[0].p, 3);                                                             // coset_idft, prover.rs:47
+}
+// The same from host evaluations: uploads a, b, c (m evaluations each, zero padded) first.
 static void enqueue_groth16_h(Engine &e, NttDomain &d, const uint64_t *a, const uint64_t *b, const uint64_t *c, size_t m) {
     const size_t n = (size_t)1 << d.k;
     const uint64_t *src[3] = {a, b, c};
@@ -1332,15 +1362,7 @@ static void enqueue_groth16_h(Engine &e, NttDomain &d, const uint64_t *a, const 
         upload_padded(e, e.ntt_buf[i].p, src[i], m, n);
     }
     CK(cudaEventRecord(e.ev[EV_H2D], e.st));
-    for (int i = 0; i < 3; i++) {
-        // idft then coset_dft (prover.rs:36-41); the 1/n and coset scalings are one elementwise pass
-        e.launches += LaunchNtt::transform(e.st, e.ntt_buf[i].p, d.inv_tw.p, d.k);
-        LaunchNtt::scale(e.st, e.ntt_buf[i].p, d.cosets.p, &d.n_inv, (uint32_t)n);
-        e.launches += 1 + LaunchNtt::transform(e.st, e.ntt_buf[i].p, d.tw.p, d.k);
-    }
-    LaunchNtt::h_pointwise(e.st, e.ntt_buf[0].p, e.ntt_buf[1].p, e.ntt_buf[2].p, &d.z_inv, (uint32_t)n);  // prover.rs:43-46
-    e.launches++;
-    ntt_enqueue(e, d, e.ntt_buf[0].p, 3);                                                             // coset_idft, prover.rs:47
+    enqueue_groth16_h_transforms(e, d, false);
 }
 
 
@@ -1368,6 +1390,13 @@ static inline size_t affine_bytes(int curve) { return curve == KGR_CURVE_BN254_G
         else if ((curve) == KGR_CURVE_BN254_G2) { CALL(Bn254G2); }         \
         else return fail(KGR_E_ARG, "unknown curve id");                   \
     } while (0)
+
+// f((C *)nullptr) for the curve type C of an id already validated (DISPATCH for code that cannot return an error code)
+template <class F> static void with_curve(int curve, F &&f) {
+    if (curve == KGR_CURVE_BN254_G1) f((Bn254G1 *)nullptr);
+    else if (curve == KGR_CURVE_GRUMPKIN) f((GrumpkinC *)nullptr);
+    else f((Bn254G2 *)nullptr);
+}
 
 }  // namespace kgr
 
@@ -2010,6 +2039,7 @@ int kgr_r1cs_register(int field, size_t m, size_t n_z, const uint32_t *const row
         s->field = field;
         s->m = m;
         s->n_z = n_z;
+        s->generation = g_generation;
         for (int k = 0; k < 3; k++) {
             size_t nnz = row_ptr[k][m];
             s->row_ptr[k].ensure(m + 1);
@@ -2279,6 +2309,148 @@ int kgr_nova_cross_term_device(kgr_r1cs_t *s, const kgr_vec_t *z1, const kgr_vec
             CK(cudaStreamSynchronize(e.st));
         }
         cudaEventElapsedTime(&s->ms[1], e.aux_ev[1], e.aux_ev[2]);
+        return KGR_OK;
+    });
+}
+
+// ---- Groth16 from the constraint system (row N1: groth16/src/prover.rs:32-65 after synthesis) ------------------------------------------------
+static int query_check(const kgr_bases *b, int curve, const char *name) {
+    if (b->curve != curve) return fail(KGR_E_ARG, std::string("the ") + name + " query must be a BN254 " + (curve == KGR_CURVE_BN254_G2 ? "G2" : "G1") + " vector");
+    if (b->generation != g_generation) return fail(KGR_E_ARG, "base handle was created before the last kgr_init");
+    if (b->shards.size() != 1 || b->shards[0].eng != 0) return fail(KGR_E_ARG, "the bases must live on the first device only (a single-device context)");
+    return KGR_OK;
+}
+
+int kgr_groth16_prove_r1cs(unsigned log_n, const kgr_r1cs_t *cs, const kgr_vec_t *z, size_t n_inputs, kgr_bases_t *h, kgr_bases_t *l, kgr_bases_t *a,
+                           kgr_bases_t *b_g1, kgr_bases_t *b_g2, uint64_t *out, uint64_t *q_out, size_t *q_len, const kgr_msm_job_t *jobs, size_t n_jobs) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (g_engines.empty()) return fail(KGR_E_NOT_INIT, "kgr_init has not been called");
+    if (!cs || !h || !l || !a || !b_g1 || !out || (!jobs && n_jobs)) return fail(KGR_E_ARG, "null pointer");
+    if (int rc = vec_check(z)) return rc;
+    if (cs->generation != g_generation) return fail(KGR_E_ARG, "R1CS shape was registered before the last kgr_init");
+    if (cs->field != 1 || z->field != 1) return fail(KGR_E_ARG, "the shape and the assignment must be over Fr (field 1)");
+    if (z->n != cs->n_z) return fail(KGR_E_ARG, "the assignment must have n_z elements (z = x ++ w)");
+    if (n_inputs == 0 || n_inputs > cs->n_z) return fail(KGR_E_ARG, "n_inputs must be in 1 .. n_z (the instance starts with the constant one)");
+    if (log_n < 1 || log_n > 28 || ((size_t)1 << log_n) < cs->m) return fail(KGR_E_ARG, "log_n must be in 1 .. 28 with 2^log_n >= m");
+    if (int rc = query_check(h, KGR_CURVE_BN254_G1, "h")) return rc;
+    if (int rc = query_check(l, KGR_CURVE_BN254_G1, "l")) return rc;
+    if (int rc = query_check(a, KGR_CURVE_BN254_G1, "a")) return rc;
+    if (int rc = query_check(b_g1, KGR_CURVE_BN254_G1, "b_g1")) return rc;
+    if (b_g2)
+        if (int rc = query_check(b_g2, KGR_CURVE_BN254_G2, "b_g2")) return rc;
+    for (size_t j = 0; j < n_jobs; j++) {
+        const kgr_msm_job_t &jb = jobs[j];
+        if (!jb.bases || !jb.out || (!jb.scalars && jb.n)) return fail(KGR_E_ARG, "null pointer");
+        if (jb.base_off > jb.bases->n || jb.n > jb.bases->n - jb.base_off) return fail(KGR_E_ARG, "range exceeds the registered vector");
+        if (jb.scalar_fmt != KGR_SCALARS_MONTGOMERY && jb.scalar_fmt != KGR_SCALARS_CANONICAL) return fail(KGR_E_ARG, "unknown scalar format");
+        if (jb.bases->curve < KGR_CURVE_BN254_G1 || jb.bases->curve > KGR_CURVE_BN254_G2) return fail(KGR_E_ARG, "unknown curve id");
+        if (int rc = query_check(jb.bases, jb.bases->curve, "job")) return rc;
+    }
+    const Params P = t_params;
+    return guarded([&]() -> int {
+        const size_t n = (size_t)1 << log_n, n_z = cs->n_z;
+        // the MSMs besides h, longest first (G2: 3x the arithmetic per point) so that the others overlap with it; pairs = zip (msm.rs:25)
+        struct Item {
+            kgr_bases *b;
+            const uint32_t *d_sc;     // scalars in z on the device, or
+            const kgr_msm_job_t *job;  // a job with host scalars
+            size_t n;
+            uint64_t *out;
+        };
+        std::vector<Item> work;
+        auto add = [&](kgr_bases *b, const uint32_t *d_sc, const kgr_msm_job_t *job, size_t pairs, uint64_t *o) {
+            if (pairs) work.push_back(Item{b, d_sc, job, pairs, o});
+            else with_curve(b->curve, [&](auto tag) { combine_partials<std::remove_pointer_t<decltype(tag)>>(std::vector<Partial>(), o); });
+        };
+        if (b_g2) add(b_g2, z->d.p, nullptr, std::min(b_g2->n, n_z), out + 48);                          // b_g2_inputs + b_g2_aux (prover.rs:64-65)
+        add(a, z->d.p, nullptr, std::min(a->n, n_z), out + 24);                                            // a_inputs + a_aux (:58-59)
+        add(b_g1, z->d.p, nullptr, std::min(b_g1->n, n_z), out + 36);                                      // b_g1_inputs + b_g1_aux (:61-62)
+        add(l, z->d.p + 8 * n_inputs, nullptr, std::min(l->n, n_z - n_inputs), out + 12);                 // l: aux only (:56)
+        for (size_t j = 0; j < n_jobs; j++) add(jobs[j].bases, nullptr, &jobs[j], jobs[j].n, jobs[j].out);
+        const size_t n_lanes = std::min(work.size() + 1, MAX_LANES);
+        ensure_lanes(0, n_lanes);
+        Engine &e0 = g_engines[0];
+        CK(cudaSetDevice(e0.dev));
+        CK(cudaEventRecord(e0.ev_input, e0.st));  // z is complete once this event is: every lane waits for it before reading z
+        auto start = [&](const Item &it, Engine &ln) {
+            with_curve(it.b->curve, [&](auto tag) {
+                typedef std::remove_pointer_t<decltype(tag)> C;
+                if (it.job) lane_start<C>(ln, P, it.b->shards[0], it.job->base_off, it.job->scalars, it.job->scalar_fmt, it.n);
+                else lane_start_device<C>(ln, P, it.b->shards[0], 0, it.d_sc, it.n, e0.ev_input);
+            });
+        };
+        auto finish = [&](const Item &it, Engine &ln) {
+            with_curve(it.b->curve, [&](auto tag) { lane_finish<std::remove_pointer_t<decltype(tag)>>(ln, it.out); });
+        };
+        // lane 0: the evaluations A z, B z, C z straight into the NTT buffers, H, then the h query on the device-resident q
+        const size_t nh = std::min(n, h->n);
+        auto h_start = [&]() {
+            Engine &e = e0;
+            e.params = P;
+            NttDomain &d = ntt_domain(e, log_n);
+            CK(cudaEventRecord(e.ev[EV_START], e.st));
+            uint32_t *bufs[3];
+            for (int i = 0; i < 3; i++) {
+                e.ntt_buf[i].ensure(n * 32);
+                bufs[i] = reinterpret_cast<uint32_t *>(e.ntt_buf[i].p);
+            }
+            LaunchR1cs::evaluate(e.st, log_n, (uint32_t)cs->m, cs->csr(0), cs->csr(1), cs->csr(2), z->d.p, bufs);
+            e.launches++;
+            CK(cudaGetLastError());
+            CK(cudaEventRecord(e.ev[EV_H2D], e.st));
+            enqueue_groth16_h_transforms(e, d, true);
+            if (nh) lane_enqueue<Bn254G1>(e, h->shards[0], 0, bufs[0], KGR_SCALARS_MONTGOMERY, nh);
+        };
+        auto h_finish = [&]() {
+            Engine &e = e0;
+            if (nh) {
+                lane_finish<Bn254G1>(e, out);
+            } else {
+                CK(cudaSetDevice(e.dev));
+                CK(cudaStreamSynchronize(e.st));
+                combine_partials<Bn254G1>(std::vector<Partial>(), out);
+            }
+            if (q_out) {
+                download_to_host(e, q_out, e.ntt_buf[0].p, n * 32, e.st);
+                if (q_len) *q_len = stripped_len(q_out, n);
+            }
+        };
+        if (!P.lane_threads) {  // one host thread (as kgr_groth16_msms): a lane that gets a second MSM finishes its first one before
+            h_start();
+            std::vector<long> pending(n_lanes, -1);
+            for (size_t j = 0; j < work.size(); j++) {
+                const size_t li = 1 + j % (n_lanes - 1);
+                if (pending[li] >= 0) finish(work[pending[li]], lane_of(0, li));
+                start(work[j], lane_of(0, li));
+                pending[li] = (long)j;
+            }
+            h_finish();
+            for (size_t li = 1; li < n_lanes; li++)
+                if (pending[li] >= 0) finish(work[pending[li]], lane_of(0, li));
+            return KGR_OK;
+        }
+        std::vector<CudaError> errs(n_lanes, CudaError{cudaSuccess, "", 0});
+        auto worker = [&](size_t li) {
+            try {
+                for (size_t j = li - 1; j < work.size(); j += n_lanes - 1) {
+                    start(work[j], lane_of(0, li));
+                    finish(work[j], lane_of(0, li));
+                }
+            } catch (CudaError &ce) {
+                errs[li] = ce;
+            }
+        };
+        std::vector<std::thread> th;
+        for (size_t li = 1; li < n_lanes; li++) th.emplace_back(worker, li);
+        try {
+            h_start();
+            h_finish();
+        } catch (CudaError &ce) {
+            errs[0] = ce;
+        }
+        for (auto &t : th) t.join();
+        for (auto &ce : errs)
+            if (ce.e != cudaSuccess) throw ce;
         return KGR_OK;
     });
 }

@@ -63,6 +63,37 @@ template <class P> KGR_HD void body_cross_term(uint32_t i, uint32_t m, const Csr
     el_store(t + 8 * (size_t)i, r);
 }
 
+// The k low bits of i reversed (fft.rs:157-162 swaps i and this index)
+KGR_HD uint32_t bitrev_k(uint32_t i, uint32_t k) {
+#ifdef __CUDA_ARCH__
+    return __brev(i) >> (32 - k);
+#else
+    uint32_t r = 0;
+    for (uint32_t b = 0; b < k; b++) r |= ((i >> b) & 1u) << (k - 1 - b);
+    return r;
+#endif
+}
+
+// cs.evaluate() (zkstd/src/r1cs.rs:137-142) straight into the three NTT buffers of the Groth16 H pipeline (groth16/src/prover.rs:36-41):
+// position i < 2^k holds row i of A z, B z, C z (zero for m <= i, the padding of prepare_fft, fft.rs:157-162) and is stored at bitrev_k(i),
+// so the first transform of each buffer starts with its butterflies.  k >= 1.
+template <class P>
+KGR_HD void body_r1cs_evaluate(uint32_t i, uint32_t k, uint32_t m, const Csr &a, const Csr &b, const Csr &c, const uint32_t *z, uint32_t *out_a,
+                               uint32_t *out_b, uint32_t *out_c) {
+    if (i >= (1u << k)) return;
+    Fp<P> r[3] = {fp_zero<P>(), fp_zero<P>(), fp_zero<P>()};
+    if (i < m) {
+        const uint32_t *zs[1] = {z};
+        row_dot<P, 1>(a, i, zs, &r[0]);
+        row_dot<P, 1>(b, i, zs, &r[1]);
+        row_dot<P, 1>(c, i, zs, &r[2]);
+    }
+    const size_t j = 8 * (size_t)bitrev_k(i, k);
+    el_store(out_a + j, r[0]);
+    el_store(out_b + j, r[1]);
+    el_store(out_c + j, r[2]);
+}
+
 // out[i] = a[i] + b[i] * r   (witness.rs:67-68)
 template <class P> KGR_HD void body_vec_fold(uint32_t i, uint32_t n, const uint32_t *a, const uint32_t *b, const Fp<P> &r, uint32_t *out) {
     if (i >= n) return;

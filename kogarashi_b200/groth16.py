@@ -10,11 +10,14 @@ Here the G1 CRS (`Parameters::{h, l, a, b_g1}`, groth16/src/params.rs:7-29) is r
 per proof the H coefficients come from the device NTT (kogarashi_b200.fft) and the `a_inputs / a_aux` and
 `b_g1_inputs / b_g1_aux` pairs are fused into one MSM each over z = inputs ++ aux (the prover splits them only because
 of its slice layout, :58-62).  The blinding terms are a five-point MSM, so no curve arithmetic is done in Python.
+`prove_r1cs` starts one step earlier, from the constraint system: the evaluations of :33 are computed on the device from a registered
+R1CS shape and the resident assignment z, and every query reads its scalars from z in device memory.
 """
 import numpy as np
 
 from .fft import Fft
-from .msm import BN254_G1, BN254_G2, SCALARS_CANONICAL, SCALARS_MONTGOMERY, Bases, groth16_msms, msm_batch, msm_curve_addition, proj_add, to_affine
+from .msm import (BN254_G1, BN254_G2, SCALARS_CANONICAL, SCALARS_MONTGOMERY, Bases, groth16_msms, groth16_prove_r1cs, msm_batch, msm_curve_addition, proj_add,
+                  to_affine)
 
 FR = 0x30644E72E131A029B85045B68181585D2833E84879B9709143E1F593F0000001  # bn254/src/fr.rs:11-16
 
@@ -64,7 +67,10 @@ class Groth16G1Prover:
                    (self.b_g1, z, 0, scalar_fmt),                   # b_g1_inputs + b_g1_aux (:61-62, :86)
                    (self.h, q, 0, scalar_fmt),                      # :51
                    (self.l, aux, 0, scalar_fmt),                    # :56
-                   (self.vk_bases, _canonical([r, 1]), 0, SCALARS_CANONICAL)]   # r*delta + alpha (:75)
+                   self._blind_a_job(r)]
+
+    def _blind_a_job(self, r):
+        return (self.vk_bases, _canonical([r, 1]), 0, SCALARS_CANONICAL)   # r*delta + alpha (:75)
 
     def _assemble_g1(self, res, r, s):
         a_answer, b1_answer, q_pt, l_pt, blind_a = res[:5]
@@ -90,6 +96,13 @@ class Groth16G1Prover:
         del jobs[2]                                                   # the h query is the fused part of the call
         q_pt, q, res = groth16_msms(log_n, a_evals, b_evals, c_evals, self.h, jobs)
         return self._assemble_g1([res[0], res[1], q_pt, res[2], res[3]], r, s) + (q,)
+
+    def prove_r1cs(self, log_n, shape, z, n_inputs, r, s):
+        """The G1 side of create_proof from the constraint system (prover.rs:32-98) in one kgr_groth16_prove_r1cs call: `shape` is the
+        nova.R1csShape of the circuit registered over FIELD_FR, `z` the nova.DeviceVec of cs.x() ++ cs.w(), the first n_inputs elements the
+        instance.  -> (A, C, q) as prove_from_evaluations."""
+        res, q, jobs = groth16_prove_r1cs(log_n, shape, z, n_inputs, self.h, self.l, self.a, self.b_g1, None, [self._blind_a_job(r)])
+        return self._assemble_g1([res["a"], res["b_g1"], res["h"], res["l"], jobs[0]], r, s) + (q,)
 
     def commitments(self, q, inputs, aux, r, s):
         """Same as prove_g1 for scalars given as Python integers."""
@@ -120,19 +133,33 @@ class Groth16Prover(Groth16G1Prover):
         All eight MSMs of prover.rs:51-65 (pairs fused) and the two independent blinding sums go to the device as one batch."""
         z, jobs = self._g1_jobs(q, inputs, aux, r, scalar_fmt)
         # the G2 query is the longest job (3x the arithmetic per point): it goes first so that the G1 queries overlap with it
-        jobs = [(self.b_g2, z, 0, scalar_fmt)] + jobs + [(self.vk_g2_bases, _canonical([s, 1]), 0, SCALARS_CANONICAL)]   # :64-65,:87 / :76
+        jobs = [(self.b_g2, z, 0, scalar_fmt)] + jobs + [self._blind_b_job(s)]   # :64-65,:87
         res = msm_batch(jobs)
         g_a, g_c = self._assemble_g1(res[1:6], r, s)
-        return g_a, to_affine(BN254_G2, proj_add(BN254_G2, res[6], res[0])), g_c
+        return g_a, self._assemble_b(res[0], res[6]), g_c
+
+    def _blind_b_job(self, s):
+        return (self.vk_g2_bases, _canonical([s, 1]), 0, SCALARS_CANONICAL)   # s*delta_g2 + beta_g2 (:76)
+
+    @staticmethod
+    def _assemble_b(b2_answer, blind_b):
+        return to_affine(BN254_G2, proj_add(BN254_G2, blind_b, b2_answer))   # :87-88
 
     def prove_from_evaluations(self, log_n, a_evals, b_evals, c_evals, inputs, aux, r, s):
         """create_proof after witness generation (prover.rs:33-98) as one kgr_groth16_msms call + the dependent blinding sum."""
         z, jobs = self._g1_jobs(np.zeros((0, 4), dtype=np.uint64), inputs, aux, r, SCALARS_MONTGOMERY)
         del jobs[2]
-        jobs = [(self.b_g2, z, 0, SCALARS_MONTGOMERY)] + jobs + [(self.vk_g2_bases, _canonical([s, 1]), 0, SCALARS_CANONICAL)]
+        jobs = [(self.b_g2, z, 0, SCALARS_MONTGOMERY)] + jobs + [self._blind_b_job(s)]
         q_pt, q, res = groth16_msms(log_n, a_evals, b_evals, c_evals, self.h, jobs)
         g_a, g_c = self._assemble_g1([res[1], res[2], q_pt, res[3], res[4]], r, s)
-        return g_a, to_affine(BN254_G2, proj_add(BN254_G2, res[5], res[0])), g_c, q
+        return g_a, self._assemble_b(res[0], res[5]), g_c, q
+
+    def prove_r1cs(self, log_n, shape, z, n_inputs, r, s):
+        """create_proof from the constraint system (prover.rs:32-98): the evaluations, H and all eight query MSMs on the device in one
+        kgr_groth16_prove_r1cs call, with the scalars read from the resident z (see Groth16G1Prover.prove_r1cs).  -> (A, B, C, q)"""
+        res, q, jobs = groth16_prove_r1cs(log_n, shape, z, n_inputs, self.h, self.l, self.a, self.b_g1, self.b_g2, [self._blind_a_job(r), self._blind_b_job(s)])
+        g_a, g_c = self._assemble_g1([res["a"], res["b_g1"], res["h"], res["l"], jobs[0]], r, s)
+        return g_a, self._assemble_b(res["b_g2"], jobs[1]), g_c, q
 
     def proof(self, q, inputs, aux, r, s):
         """Scalars as Python integers."""

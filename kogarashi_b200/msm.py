@@ -161,6 +161,23 @@ def groth16_msms(log_n, a_evals, b_evals, c_evals, h_bases, jobs, scalar_fmt=SCA
     return h_out, (q[: q_len.value] if want_q else None), outs
 
 
+def groth16_prove_r1cs(log_n, shape, z, n_inputs, h, l, a, b_g1, b_g2, jobs, want_q=True):
+    """kgr_groth16_prove_r1cs: prover.rs:32-65 from a registered R1CS shape (nova.R1csShape over Fr) and the resident assignment z = x ++ w
+    (nova.DeviceVec; x = the n_inputs instance elements, the constant one first).  b_g2 may be None (G1 only); `jobs` as in msm_batch.
+    -> ({"h", "l", "a", "b_g1"[, "b_g2"]: projective results}, q (stripped) or None, [job results])."""
+    _lib.ensure_init()
+    arr, keep, outs = _job_array(jobs, SCALARS_MONTGOMERY)
+    out = np.zeros(72, dtype=np.uint64)
+    q = np.zeros((1 << log_n, 4), dtype=np.uint64) if want_q else None
+    q_len = ctypes.c_size_t()
+    _lib.check(_lib.lib().kgr_groth16_prove_r1cs(log_n, shape._h, z._h, n_inputs, h._h, l._h, a._h, b_g1._h, b_g2._h if b_g2 is not None else None,
+                                                 _u64(out), _u64(q) if want_q else None, ctypes.byref(q_len), ctypes.cast(arr, ctypes.c_void_p), len(jobs)))
+    res = {"h": out[0:12], "l": out[12:24], "a": out[24:36], "b_g1": out[36:48]}
+    if b_g2 is not None:
+        res["b_g2"] = out[48:72]
+    return res, (q[: q_len.value] if want_q else None), outs
+
+
 def msm_device(bases, d_scalars_ptr, n, scalar_fmt=SCALARS_MONTGOMERY, base_off=0):
     """MSM with the scalars already in device memory (raw pointer, n x 4 uint64)."""
     out = np.zeros(3 * coord_limbs(bases.curve), dtype=np.uint64)

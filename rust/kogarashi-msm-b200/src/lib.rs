@@ -79,6 +79,9 @@ extern "C" {
     fn kgr_host_free(p: *mut c_void) -> i32;
     fn kgr_groth16_msms(log_n: u32, a: *const u64, b: *const u64, c: *const u64, m: usize, h: *mut kgr_bases_t, h_out: *mut u64, q_out: *mut u64,
                         q_len: *mut usize, jobs: *const kgr_msm_job_t, n_jobs: usize) -> i32;
+    fn kgr_groth16_prove_r1cs(log_n: u32, cs: *const kgr_r1cs_t, z: *const kgr_vec_t, n_inputs: usize, h: *mut kgr_bases_t, l: *mut kgr_bases_t,
+                              a: *mut kgr_bases_t, b_g1: *mut kgr_bases_t, b_g2: *mut kgr_bases_t, out: *mut u64, q_out: *mut u64, q_len: *mut usize,
+                              jobs: *const kgr_msm_job_t, n_jobs: usize) -> i32;
     fn kgr_set_param(name: *const c_char, value: c_long) -> i32;
     fn kgr_last_timing(dev: i32, ms: *mut f32, shape: *mut u32) -> i32;
     fn kgr_event_record(dev: i32, idx: i32) -> i32;
@@ -373,6 +376,22 @@ impl GpuProver {
         use bn_254::{G1Affine, G2Affine};
         ProverQueries { q: G1Affine::extended_from_limbs(&oh), l: G1Affine::extended_from_limbs(&ol), a_answer: G1Affine::extended_from_limbs(&oa),
                         b1_answer: G1Affine::extended_from_limbs(&ob1), b2_answer: G2Affine::extended_from_limbs(&ob2) }
+    }
+
+    /// prover.rs:32-65 in one `kgr_groth16_prove_r1cs` call, straight after synthesis: `cs.evaluate()` on the device from the registered shape
+    /// (`R1csShapeGpu` over Fr, columns `Wire::Instance(i) -> i`, `Wire::Witness(i) -> n_inputs + i`), H, and every query with its scalars read
+    /// from the resident `z = cs.x() ++ cs.w()` (`DeviceVec` over Fr; `n_inputs = cs.x().len()`, the constant one first).  The blinding sums of
+    /// :75-92 stay with the caller, as after `queries`.
+    pub fn prove_r1cs(&self, log_n: u32, cs: &R1csShapeGpu, z: &DeviceVec, n_inputs: usize) -> ProverQueries {
+        let mut out = [0u64; 72];
+        check(unsafe {
+            kgr_groth16_prove_r1cs(log_n, cs.handle, z.handle, n_inputs, self.h.handle, self.l.handle, self.a.handle, self.b_g1.handle, self.b_g2.handle,
+                                   out.as_mut_ptr(), core::ptr::null_mut(), core::ptr::null_mut(), core::ptr::null(), 0)
+        });
+        use bn_254::{G1Affine, G2Affine};
+        ProverQueries { q: G1Affine::extended_from_limbs(&out[0..12]), l: G1Affine::extended_from_limbs(&out[12..24]),
+                        a_answer: G1Affine::extended_from_limbs(&out[24..36]), b1_answer: G1Affine::extended_from_limbs(&out[36..48]),
+                        b2_answer: G2Affine::extended_from_limbs(&out[48..72]) }
     }
 }
 
