@@ -6,18 +6,18 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = os.path.join(ROOT, "tests", "_build", "abi_demo")
 
 
 @pytest.fixture(scope="module")
-def demo():
+def demo(tmp_path_factory):
+    """The demo program, built into a temporary directory: the source tree may be read-only."""
     from kogarashi_b200 import _lib
     _lib.build()
-    os.makedirs(os.path.dirname(EXE), exist_ok=True)
+    exe = str(tmp_path_factory.mktemp("abi_demo") / "abi_demo")
     libdir = os.path.join(ROOT, "kogarashi_b200")
-    subprocess.check_call(["gcc", "-O2", "-Wall", "-Werror", "-I", os.path.join(ROOT, "include"), "-o", EXE, os.path.join(ROOT, "examples", "abi_demo.c"),
+    subprocess.check_call(["gcc", "-O2", "-Wall", "-Werror", "-I", os.path.join(ROOT, "include"), "-o", exe, os.path.join(ROOT, "examples", "abi_demo.c"),
                            "-L", libdir, "-lkgr_msm", f"-Wl,-rpath,{libdir}"])
-    return EXE
+    return exe
 
 
 def test_header_compiles_as_c_and_program_fails_loudly_without_a_device(demo):

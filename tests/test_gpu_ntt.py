@@ -14,7 +14,7 @@ def k():
     return kk
 
 
-@pytest.mark.parametrize("log_n", [1, 2, 3, 5, 8, 10, 11, 13, 16])
+@pytest.mark.parametrize("log_n", [1, 2, 3, 5, 8, 10, 11, 13, 16, 20])  # 20: the largest two-pass domain (10 + 10 stages)
 def test_transforms_bit_exact(k, log_n):
     n = 1 << log_n
     f = k.Fft(log_n)
@@ -57,14 +57,15 @@ def test_fft_multiplication_matches_naive(k):
     assert got.shape[0] == 2 * d - 1 and (got == naive).all()
 
 
-@pytest.mark.parametrize("log_n,m", [(2, 4), (10, 1000), (14, 1 << 14)])
+# 2^21 and 2^22 run three passes per transform; m = n / 2 + 1 is mostly padding
+@pytest.mark.parametrize("log_n,m", [(2, 4), (10, 1000), (14, 1 << 14), (21, 1 << 21), (21, (1 << 20) + 1), (22, 1 << 22), (22, (1 << 21) + 1)])
 def test_h_coefficients_match_reference_pipeline(k, log_n, m):
     """prover.rs:36-47 on the device == the same pipeline through the restated reference FFT."""
     f = k.Fft(log_n)
     a = A.random_field(A.FIELD_FR, m, seed=bytes(range(3, 19)))
     b = A.random_field(A.FIELD_FR, m, seed=bytes(range(4, 20)))
     # make c = a * b on the domain so that H is a genuine quotient (degree <= n - 2)
-    c = np.stack([A.field_op(A.FIELD_FR, "mul", a[i], b[i]) for i in range(m)])
+    c = A.sparse_prod(A.FIELD_FR, m, (np.arange(m + 1, dtype=np.uint32), np.arange(m, dtype=np.uint32), a), b)  # diag(a) b
     exp, n_exp = A.groth16_h(log_n, a, b, c)
     got = f.h_coefficients(a, b, c)
     assert got.shape[0] == n_exp and (got == exp[:n_exp]).all()
