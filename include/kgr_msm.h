@@ -199,6 +199,27 @@ int kgr_groth16_msms(unsigned log_n, const uint64_t *a, const uint64_t *b, const
 int kgr_groth16_prove_r1cs(unsigned log_n, const kgr_r1cs_t *cs, const kgr_vec_t *z, size_t n_inputs, kgr_bases_t *h, kgr_bases_t *l, kgr_bases_t *a,
                            kgr_bases_t *b_g1, kgr_bases_t *b_g2, uint64_t *out, uint64_t *q_out, size_t *q_len, const kgr_msm_job_t *jobs, size_t n_jobs);
 
+/* groth16/src/zksnark.rs:17-127 (ZkSnark::setup) on the device, from a shape registered over Fr (field 1) and its number of instance variables
+ * (the constant one included, z = x ++ w as kgr_groth16_prove_r1cs).  toxic: alpha, beta, gamma, delta, tau, 4 x u64 Montgomery each (< r).
+ * With n = 2^k, k = max(1, ceil(log2 m)), l_i = L_i(tau) over that domain and u_j, v_j, w_j = sum_i A/B/C[i][j] * l_i:
+ *   a_j = u_j * G1   b_g1_j = v_j * G1   b_g2_j = v_j * G2   ic_j (j < n_inputs) = (beta u_j + alpha v_j + w_j) / gamma * G1
+ *   l_j (j >= n_inputs) = (beta u_j + alpha v_j + w_j) / delta * G1   h_i = tau^i (tau^n - 1) / delta * G1 for i < m - 1
+ * Outputs are new single-shard handles on the first device, ready for kgr_groth16_prove_r1cs:
+ *   a, b_g1, b_g2: n_z points   ic: n_inputs   l: n_z - n_inputs   h: m - 1   (the identity, stored (0, 0), where the exponent is 0)
+ * vk_g1: alpha, beta, delta (3 x 9: x[4] y[4] is_infinity);  vk_g2: beta, gamma, delta (3 x 17); an identity reads (0, 0, 1).
+ * *log_n_out = k.  b_g2 == NULL: no G2 query is built (vk_g2 may then be NULL too; it is filled whenever it is given).
+ * The h query has m - 1 entries, as the reference builds it.  H = (AB - C) / Z has up to n - 1 coefficients, so for m < 2^k a proof can need
+ * entries the query lacks: proofs are guaranteed valid for m = 2^k only.
+ * Refused with KGR_E_ARG before any work, every output handle left NULL: a NULL required pointer, a shape registered before the last kgr_init,
+ * a shape over Fq, n_inputs == 0 or > n_z, k > 28, toxic values >= r, gamma == 0 or delta == 0, a context of more than one device.
+ * On a later failure everything allocated is freed. */
+int kgr_groth16_setup(const kgr_r1cs_t *cs, size_t n_inputs, const uint64_t toxic[20], uint32_t *log_n_out, kgr_bases_t **h, kgr_bases_t **l,
+                      kgr_bases_t **a, kgr_bases_t **b_g1, kgr_bases_t **b_g2, kgr_bases_t **ic, uint64_t *vk_g1, uint64_t *vk_g2);
+/* Device time (ms, CUDA events) of the phases of the last kgr_groth16_setup: [0] powers of tau + idft, [1] column index + sums of A, B, C,
+ * [2] scalars, fixed-base multiplications of [3] a, [4] b_g1, [5] ic, [6] l, [7] h, [8] b_g2, [9] vk.  The one-time NTT and generator tables
+ * of a device are built before [0] and are not included. */
+int kgr_groth16_setup_last_timing(float ms[10]);
+
 /* Tuning knobs: "window_bits" (0 = auto), "chunk" (entries per accumulate thread, 0 = auto),
  * "reduce_fanin" (power of two), "running_sum_stop" (elements per window below which the reduce
  * switches from running sums to the parallel weighting pass), "final_on_device" (1: Horner over

@@ -19,7 +19,7 @@ EXPORTS = [
     "kgr_fixed_base_mul", "kgr_bases_generate", "kgr_microbench", "kgr_bases_download", "kgr_event_record",
     "kgr_event_elapsed_ms", "kgr_launch_count", "kgr_bases_precompute", "kgr_ntt", "kgr_ntt_device", "kgr_groth16_h",
     "kgr_bases_generate_at", "kgr_vec_upload", "kgr_vec_download", "kgr_vec_free", "kgr_vec_len", "kgr_vec_write", "kgr_vec_fold_device", "kgr_msm_vec",
-    "kgr_pedersen_commit_vec", "kgr_nova_cross_term_device", "kgr_host_alloc", "kgr_host_free", "kgr_msm_batch", "kgr_groth16_msms", "kgr_groth16_prove_r1cs", "kgr_r1cs_register", "kgr_r1cs_free", "kgr_r1cs_mul", "kgr_nova_cross_term", "kgr_r1cs_last_timing", "kgr_vec_fold",
+    "kgr_pedersen_commit_vec", "kgr_nova_cross_term_device", "kgr_host_alloc", "kgr_host_free", "kgr_msm_batch", "kgr_groth16_msms", "kgr_groth16_prove_r1cs", "kgr_groth16_setup", "kgr_groth16_setup_last_timing", "kgr_r1cs_register", "kgr_r1cs_free", "kgr_r1cs_mul", "kgr_nova_cross_term", "kgr_r1cs_last_timing", "kgr_vec_fold",
 ]
 
 
@@ -82,6 +82,8 @@ def lib():
     L.kgr_msm_batch.argtypes = [vp, sz]
     L.kgr_groth16_msms.argtypes = [ctypes.c_uint, u64p, u64p, u64p, sz, vp, u64p, u64p, ctypes.POINTER(sz), vp, sz]
     L.kgr_groth16_prove_r1cs.argtypes = [ctypes.c_uint, vp, vp, sz, vp, vp, vp, vp, vp, u64p, u64p, ctypes.POINTER(sz), vp, sz]
+    L.kgr_groth16_setup.argtypes = [vp, sz, u64p, ctypes.POINTER(ctypes.c_uint32)] + [ctypes.POINTER(vp)] * 6 + [u64p, u64p]
+    L.kgr_groth16_setup_last_timing.argtypes = [ctypes.POINTER(ctypes.c_float)]
     L.kgr_r1cs_free.argtypes = [vp]
     L.kgr_r1cs_mul.argtypes = [vp, ci, u64p, u64p]
     L.kgr_nova_cross_term.argtypes = [vp, u64p, u64p, u64p, vp, u64p]

@@ -110,4 +110,18 @@ struct LaunchR1cs {
     static void evaluate(cudaStream_t st, uint32_t k, uint32_t m, const Csr &a, const Csr &b, const Csr &c, const uint32_t *z, uint32_t *const out[3]);
 };
 
+// Groth16 parameter generation over Fr (kernels_setup.cu, bodies in setup_kernels.cuh).  Each returns the kernels it launched.
+struct LaunchSetup {
+    // tau^i for i < 2^k from lo[j] = tau^j (j < 2^tau_log_t(k)) and hi[b] = tau^(2^tau_log_t(k) * b); out[0 .. n_h) is copied to h
+    static uint32_t tau_log_t(uint32_t k) { return (k + 1) / 2; }
+    static int tau_powers(cudaStream_t st, uint32_t k, const void *lo, const void *hi, void *out, uint32_t n_h, void *h);
+    // out[j] = sum over the entries (i, j) of mat of coeff * lagr[i], j < n_z.  cnt: n_z + 1 words, zero on entry; ptr[0..1]: n_z + 1 words each;
+    // vals[0..1]: nnz elements each; tile_sums: LaunchUtil::scan_tiles(n_z + 1) words
+    static int column_sums(cudaStream_t st, uint32_t m, uint32_t n_z, const Csr &mat, uint32_t nnz, const void *lagr, uint32_t *cnt, uint32_t *const ptr[2],
+                           void *const vals[2], uint32_t *tile_sums, void *out);
+    // consts: alpha, beta, 1/gamma, 1/delta, (tau^n - 1)/delta (setup_kernels.cuh: SetupConsts); ext: n_z elements; h: n_h elements, tau^i on entry
+    static int scalars(cudaStream_t st, uint32_t n_z, uint32_t n_inputs, uint32_t n_h, const void *consts, const void *u, const void *v, const void *w,
+                       void *ext, void *h);
+};
+
 }  // namespace kgr

@@ -35,6 +35,7 @@
 #include "../../include/kgr_msm.h"
 #include "launch.cuh"
 #include "r1cs_kernels.cuh"
+#include "setup_kernels.cuh"
 
 namespace kgr {
 
@@ -815,7 +816,8 @@ struct kgr_bases {
 struct kgr_r1cs {
     int field = 0;
     size_t m = 0, n_z = 0;
-    uint64_t generation = 0;  // kgr_init that created it (checked by kgr_groth16_prove_r1cs)
+    uint64_t generation = 0;  // kgr_init that created it (checked by kgr_groth16_prove_r1cs and kgr_groth16_setup)
+    size_t nnz[3] = {0, 0, 0};
     kgr::DevBuf<uint32_t> row_ptr[3], cols[3], coeffs[3], z1, z2, t;
     float ms[3] = {0, 0, 0};  // last cross term: H2D of z1 / z2, kernel, commit MSM
     kgr::Csr csr(int i) const { return kgr::Csr{row_ptr[i].p, cols[i].p, coeffs[i].p}; }
@@ -1247,6 +1249,25 @@ template <class C> static void generate_shard(Engine &e, Shard &s, uint64_t seed
     CK(cudaStreamSynchronize(e.st));
     if (k_out) CK(cudaMemcpy(k_out + 4 * s.first, dk, s.count * sizeof(S), cudaMemcpyDeviceToHost));
     CK(cudaFree(dk));
+}
+
+// A new single-shard handle on engine e holding k[i] * G for i < n (device scalars, Montgomery): a zero scalar gives (0, 0), the identity as
+// registered handles store it (k_fold_inf).
+template <class C> static std::unique_ptr<kgr_bases> fixed_base_handle(Engine &e, int curve, const void *d_k, size_t n) {
+    std::unique_ptr<kgr_bases> b(new kgr_bases);
+    b->curve = curve;
+    b->n = n;
+    b->generation = g_generation;
+    make_shards(b->shards, n);
+    Shard &s = b->shards[0];
+    s.dev = e.dev;
+    CK(cudaMalloc(&s.d_pts, std::max<size_t>(n, 1) * sizeof(AffinePt<C>)));
+    if (n) {
+        Launch<C>::fixed_base(e.st, (const Fp<typename C::Scalar> *)d_k, fixed_table<C>(e), (uint32_t)n, (AffinePt<C> *)s.d_pts);
+        e.launches++;
+        CK(cudaGetLastError());
+    }
+    return b;
 }
 
 static double ubench_mode(Engine &e, int mode, uint32_t *sink, double ops_per_thread_iter) {
@@ -2042,6 +2063,7 @@ int kgr_r1cs_register(int field, size_t m, size_t n_z, const uint32_t *const row
         s->generation = g_generation;
         for (int k = 0; k < 3; k++) {
             size_t nnz = row_ptr[k][m];
+            s->nnz[k] = nnz;
             s->row_ptr[k].ensure(m + 1);
             s->cols[k].ensure(std::max<size_t>(nnz, 1));
             s->coeffs[k].ensure(std::max<size_t>(nnz, 1) * 8);
@@ -2453,6 +2475,161 @@ int kgr_groth16_prove_r1cs(unsigned log_n, const kgr_r1cs_t *cs, const kgr_vec_t
             if (ce.e != cudaSuccess) throw ce;
         return KGR_OK;
     });
+}
+
+// ---- Groth16 parameter generation (groth16/src/zksnark.rs:17-127) on the device ---------------------------------------------------------
+static float g_setup_ms[10] = {};  // phases of the last kgr_groth16_setup (kgr_groth16_setup_last_timing)
+
+static bool fr_canonical(const uint64_t *w) {  // w < r: the field code takes fully reduced residues only
+    for (int i = 3; i >= 0; i--) {
+        const uint64_t r = ((uint64_t)FrP::mod(2 * i + 1) << 32) | FrP::mod(2 * i);
+        if (w[i] != r) return w[i] < r;
+    }
+    return false;
+}
+
+int kgr_groth16_setup(const kgr_r1cs_t *cs, size_t n_inputs, const uint64_t toxic[20], uint32_t *log_n_out, kgr_bases_t **h, kgr_bases_t **l,
+                      kgr_bases_t **a, kgr_bases_t **b_g1, kgr_bases_t **b_g2, kgr_bases_t **ic, uint64_t *vk_g1, uint64_t *vk_g2) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    for (kgr_bases_t **o : {h, l, a, b_g1, b_g2, ic})
+        if (o) *o = nullptr;
+    if (g_engines.empty()) return fail(KGR_E_NOT_INIT, "kgr_init has not been called");
+    if (!cs || !toxic || !log_n_out || !h || !l || !a || !b_g1 || !ic || !vk_g1 || (b_g2 && !vk_g2)) return fail(KGR_E_ARG, "null pointer");
+    if (cs->generation != g_generation) return fail(KGR_E_ARG, "R1CS shape was registered before the last kgr_init");
+    if (cs->field != 1) return fail(KGR_E_ARG, "the shape must be over Fr (field 1)");
+    if (n_inputs == 0 || n_inputs > cs->n_z) return fail(KGR_E_ARG, "n_inputs must be in 1 .. n_z (the instance starts with the constant one)");
+    uint32_t k = 1;
+    while (((size_t)1 << k) < cs->m) k++;
+    if (k > 28) return fail(KGR_E_ARG, "m exceeds 2^28, the largest Fr domain");
+    for (int i = 0; i < 5; i++)
+        if (!fr_canonical(toxic + 4 * i)) return fail(KGR_E_ARG, "toxic waste must be reduced modulo r");
+    for (int i : {2, 3})
+        if (!(toxic[4 * i] | toxic[4 * i + 1] | toxic[4 * i + 2] | toxic[4 * i + 3])) return fail(KGR_E_ARG, "gamma and delta must be non-zero");
+    if (g_engines.size() != 1) return fail(KGR_E_ARG, "setup needs a single-device context (the queries live on the first device, unsplit)");
+    return guarded([&]() -> int {
+        Engine &e = g_engines[0];
+        CK(cudaSetDevice(e.dev));
+        const size_t n = (size_t)1 << k, n_z = cs->n_z, n_h = cs->m ? cs->m - 1 : 0;
+        Fp<FrP> t[5];  // alpha, beta, gamma, delta, tau
+        for (int i = 0; i < 5; i++) std::memcpy(&t[i], toxic + 4 * i, 32);
+        const Fp<FrP> &tau = t[4];
+        SetupConsts<FrP> consts{t[0], t[1], fp_inv(t[2]), fp_inv(t[3]), fp_zero<FrP>()};
+        consts.h_coeff = fp_mul(fp_sub(fr_pow2k(tau, k), fp_one<FrP>()), consts.delta_inv);  // (tau^n - 1) / delta (zksnark.rs:52-53)
+        const uint32_t log_t = LaunchSetup::tau_log_t(k);
+        const Fp<FrP> tau_t = fr_pow2k(tau, log_t);
+        const size_t nnz_max = std::max({cs->nnz[0], cs->nnz[1], cs->nnz[2], (size_t)1});
+        struct Scratch {
+            DevBuf<uint8_t> lo, hi, lagr, hs, uvw[3], ext, vals[2], vk_k, vk_pts;
+            DevBuf<uint32_t> cnt, ptr[2], tile_sums;
+            ~Scratch() {
+                for (auto *b : {&lo, &hi, &lagr, &hs, &uvw[0], &uvw[1], &uvw[2], &ext, &vals[0], &vals[1], &vk_k, &vk_pts}) b->release();
+                for (auto *b : {&cnt, &ptr[0], &ptr[1], &tile_sums}) b->release();
+            }
+        } sc;
+        sc.lo.ensure(((size_t)1 << log_t) * 32);
+        sc.hi.ensure((n >> log_t) * 32);
+        sc.lagr.ensure(n * 32);
+        sc.hs.ensure(std::max<size_t>(n_h, 1) * 32);
+        for (auto &b : sc.uvw) b.ensure(n_z * 32);
+        sc.ext.ensure(n_z * 32);
+        for (auto &b : sc.vals) b.ensure(nnz_max * 32);
+        sc.cnt.ensure(n_z + 1);
+        for (auto &b : sc.ptr) b.ensure(n_z + 1);
+        sc.tile_sums.ensure(LaunchUtil::scan_tiles((uint32_t)n_z + 1));
+        sc.vk_k.ensure(6 * 32);
+        sc.vk_pts.ensure(3 * sizeof(AffinePt<Bn254G1>) + 3 * sizeof(AffinePt<Bn254G2>));
+        // vk scalars: alpha, beta, delta (G1) then beta, gamma, delta (G2)
+        const Fp<FrP> vk_k[6] = {t[0], t[1], t[3], t[1], t[2], t[3]};
+        CK(cudaMemcpyAsync(sc.vk_k.p, vk_k, sizeof vk_k, cudaMemcpyHostToDevice, e.st));
+        // one-time tables (cached per engine), outside the timed phases
+        NttDomain &d = ntt_domain(e, k);
+        fixed_table<Bn254G1>(e);
+        if (b_g2 || vk_g2) fixed_table<Bn254G2>(e);
+        cudaEvent_t ev[11] = {};
+        struct Events {
+            cudaEvent_t *ev;
+            ~Events() {
+                for (int i = 0; i < 11; i++)
+                    if (ev[i]) cudaEventDestroy(ev[i]);
+            }
+        } ev_guard{ev};
+        for (auto &x : ev) CK(cudaEventCreate(&x));
+        int mark = 0;
+        auto phase = [&]() { CK(cudaEventRecord(ev[mark++], e.st)); };
+        phase();
+        // powers of tau (the first m - 1 also into h, zksnark.rs:51-57), then the Lagrange basis at tau = idft of the powers (zksnark.rs:60)
+        LaunchNtt::pow_table(e.st, sc.lo.p, &tau, 1u << log_t);
+        LaunchNtt::pow_table(e.st, sc.hi.p, &tau_t, (uint32_t)(n >> log_t));
+        e.launches += 2 + LaunchSetup::tau_powers(e.st, k, sc.lo.p, sc.hi.p, sc.lagr.p, (uint32_t)n_h, sc.hs.p);
+        ntt_enqueue(e, d, sc.lagr.p, 1);
+        CK(cudaGetLastError());
+        phase();
+        // u, v, w per variable (zksnark.rs:62-87: eval_at_tau of the columns of A, B, C)
+        uint32_t *ptr[2] = {sc.ptr[0].p, sc.ptr[1].p};
+        for (int i = 0; i < 3; i++) {
+            void *vals[2] = {sc.vals[0].p, sc.vals[1].p};
+            CK(cudaMemsetAsync(sc.cnt.p, 0, (n_z + 1) * sizeof(uint32_t), e.st));
+            e.launches += LaunchSetup::column_sums(e.st, (uint32_t)cs->m, (uint32_t)n_z, cs->csr(i), (uint32_t)cs->nnz[i], sc.lagr.p, sc.cnt.p, ptr, vals,
+                                                   sc.tile_sums.p, sc.uvw[i].p);
+            CK(cudaGetLastError());
+        }
+        phase();
+        e.launches += LaunchSetup::scalars(e.st, (uint32_t)n_z, (uint32_t)n_inputs, (uint32_t)n_h, &consts, sc.uvw[0].p, sc.uvw[1].p, sc.uvw[2].p, sc.ext.p,
+                                           sc.hs.p);
+        CK(cudaGetLastError());
+        phase();
+        // the queries: a_j = u_j, b_j = v_j, ic / l from ext, h (zksnark.rs:51-87)
+        std::unique_ptr<kgr_bases> qa = fixed_base_handle<Bn254G1>(e, KGR_CURVE_BN254_G1, sc.uvw[0].p, n_z);
+        phase();
+        std::unique_ptr<kgr_bases> qb1 = fixed_base_handle<Bn254G1>(e, KGR_CURVE_BN254_G1, sc.uvw[1].p, n_z);
+        phase();
+        std::unique_ptr<kgr_bases> qic = fixed_base_handle<Bn254G1>(e, KGR_CURVE_BN254_G1, sc.ext.p, n_inputs);
+        phase();
+        std::unique_ptr<kgr_bases> ql = fixed_base_handle<Bn254G1>(e, KGR_CURVE_BN254_G1, sc.ext.p + 32 * n_inputs, n_z - n_inputs);
+        phase();
+        std::unique_ptr<kgr_bases> qh = fixed_base_handle<Bn254G1>(e, KGR_CURVE_BN254_G1, sc.hs.p, n_h);
+        phase();
+        std::unique_ptr<kgr_bases> qb2;
+        if (b_g2) qb2 = fixed_base_handle<Bn254G2>(e, KGR_CURVE_BN254_G2, sc.uvw[1].p, n_z);
+        phase();
+        AffinePt<Bn254G1> *vk1 = (AffinePt<Bn254G1> *)sc.vk_pts.p;
+        AffinePt<Bn254G2> *vk2 = (AffinePt<Bn254G2> *)(vk1 + 3);
+        Launch<Bn254G1>::fixed_base(e.st, (const Fp<FrP> *)sc.vk_k.p, fixed_table<Bn254G1>(e), 3, vk1);
+        e.launches++;
+        if (vk_g2) {
+            Launch<Bn254G2>::fixed_base(e.st, (const Fp<FrP> *)sc.vk_k.p + 3, fixed_table<Bn254G2>(e), 3, vk2);
+            e.launches++;
+        }
+        CK(cudaGetLastError());
+        phase();
+        uint64_t pts[3 * 8 + 3 * 16];
+        CK(cudaMemcpyAsync(pts, sc.vk_pts.p, sizeof pts, cudaMemcpyDeviceToHost, e.st));
+        CK(cudaStreamSynchronize(e.st));
+        for (int i = 0; i < 10; i++) CK(cudaEventElapsedTime(&g_setup_ms[i], ev[i], ev[i + 1]));
+        auto put = [](const uint64_t *xy, int words, uint64_t *o) {  // x y is_infinity; the identity reads (0, 0, 1) as in kgr_bases_download
+            uint64_t any = 0;
+            for (int w = 0; w < words; w++) any |= (o[w] = xy[w]);
+            o[words] = any ? 0 : 1;
+        };
+        for (int i = 0; i < 3; i++) put(pts + 8 * i, 8, vk_g1 + 9 * i);
+        if (vk_g2)
+            for (int i = 0; i < 3; i++) put(pts + 24 + 16 * i, 16, vk_g2 + 17 * i);
+        *log_n_out = k;
+        *a = qa.release();
+        *b_g1 = qb1.release();
+        *ic = qic.release();
+        *l = ql.release();
+        *h = qh.release();
+        if (b_g2) *b_g2 = qb2.release();
+        return KGR_OK;
+    });
+}
+
+int kgr_groth16_setup_last_timing(float ms[10]) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (!ms) return fail(KGR_E_ARG, "null pointer");
+    std::memcpy(ms, g_setup_ms, sizeof g_setup_ms);
+    return KGR_OK;
 }
 
 int kgr_host_alloc(size_t bytes, void **out) {

@@ -12,12 +12,16 @@ per proof the H coefficients come from the device NTT (kogarashi_b200.fft) and t
 of its slice layout, :58-62).  The blinding terms are a five-point MSM, so no curve arithmetic is done in Python.
 `prove_r1cs` starts one step earlier, from the constraint system: the evaluations of :33 are computed on the device from a registered
 R1CS shape and the resident assignment z, and every query reads its scalars from z in device memory.
+`setup` generates the parameters themselves (groth16/src/zksnark.rs:17-127) on the device from the registered shape; `from_params` hands its
+resident queries to a prover without a download or a re-upload.
 """
+import os
+
 import numpy as np
 
 from .fft import Fft
-from .msm import (BN254_G1, BN254_G2, SCALARS_CANONICAL, SCALARS_MONTGOMERY, Bases, groth16_msms, groth16_prove_r1cs, msm_batch, msm_curve_addition, proj_add,
-                  to_affine)
+from .msm import (BN254_G1, BN254_G2, SCALARS_CANONICAL, SCALARS_MONTGOMERY, Bases, coord_limbs, groth16_msms, groth16_prove_r1cs, groth16_setup,
+                  msm_batch, msm_curve_addition, proj_add, to_affine)
 
 FR = 0x30644E72E131A029B85045B68181585D2833E84879B9709143E1F593F0000001  # bn254/src/fr.rs:11-16
 
@@ -44,6 +48,70 @@ def _canonical(vals):
     return out
 
 
+def _mont(vals):
+    return _canonical([v * (1 << 256) for v in vals])
+
+
+class Groth16Params:
+    """The parameters of zksnark.rs:17-127 with every query resident on the device (`setup`): `a`, `b_g1`, `b_g2` (None for a G1-only setup),
+    `ic`, `l`, `h` are `Bases`; `vk_g1` (3, 9) holds alpha, beta, delta and `vk_g2` (3, 17) beta, gamma, delta as x, y, is_infinity.
+    `log_n` is the domain the prover must use.  The h query has m - 1 entries as in the reference, so a proof is only guaranteed to be valid
+    for m = 2^log_n.  A prover built with `from_params` takes over a, b_g1, h, l (and b_g2) and frees them; `ic` and the vk stay here."""
+
+    QUERIES = ("a", "b_g1", "b_g2", "ic", "l", "h")
+
+    def __init__(self, log_n, queries, vk_g1, vk_g2):
+        self.log_n, self.vk_g1, self.vk_g2 = log_n, vk_g1, vk_g2
+        for name in self.QUERIES:
+            setattr(self, name, queries.get(name))
+
+    def take(self, *names):
+        """Hand the named query handles over to a new owner: they are no longer held (or freed) by these parameters."""
+        out = []
+        for name in names:
+            b = getattr(self, name)
+            if b is None:
+                raise ValueError(f"the {name} query is not held by these parameters (not generated, or already taken)")
+            setattr(self, name, None)
+            out.append(b)
+        return out
+
+    def download(self):
+        """-> {"log_n", "vk_g1", "vk_g2", and per query still held: (points (n, 8) or (n, 16) uint64 Montgomery x || y, is_infinity (n,) uint8)}:
+        the host arrays for serialisation and for a verifier (an identity reads (0, 0) with its flag set)."""
+        out = dict(log_n=self.log_n, vk_g1=self.vk_g1.copy(), vk_g2=None if self.vk_g2 is None else self.vk_g2.copy())
+        for name in self.QUERIES:
+            b = getattr(self, name)
+            if b is not None:
+                pts = b.download() if b.n else np.zeros((0, 2 * coord_limbs(b.curve)), dtype=np.uint64)
+                out[name] = (pts, (~pts.any(axis=1)).astype(np.uint8))
+        return out
+
+    def free(self):
+        for name in self.QUERIES:
+            b = getattr(self, name)
+            if b is not None:
+                b.free()
+                setattr(self, name, None)
+
+
+def setup(shape, n_inputs, toxic=None, g2=True):
+    """ZkSnark::setup (groth16/src/zksnark.rs:17-127) on the device: `shape` is the nova.R1csShape of the circuit registered over FIELD_FR with
+    columns over z = x ++ w, `n_inputs` = len(x) (the constant one included).  toxic: (alpha, beta, gamma, delta, tau) as Python ints; by default
+    each is 64 bytes of os.urandom reduced modulo r, redrawn while zero.  g2=False skips the G2 query.  -> Groth16Params"""
+    if toxic is None:
+        toxic = []
+        while len(toxic) < 5:
+            v = int.from_bytes(os.urandom(64), "little") % FR
+            if v:
+                toxic.append(v)
+    toxic = [int(v) % FR for v in toxic]
+    if len(toxic) != 5:
+        raise ValueError("toxic waste is five field elements: alpha, beta, gamma, delta, tau")
+    log_n, queries, vk_g1, vk_g2 = groth16_setup(shape, n_inputs, _mont(toxic), g2)
+    return Groth16Params(log_n, queries, vk_g1, vk_g2)
+
+
 class Groth16G1Prover:
     """Points are (n, 8) uint64 Montgomery arrays with (n,) uint8 infinity flags (CRS entries may be the identity,
     groth16/src/zksnark.rs:62-66,177-185)."""
@@ -51,10 +119,29 @@ class Groth16G1Prover:
     def __init__(self, delta_g1, alpha_g1, beta_g1, a, a_inf, b_g1, b_g1_inf, h, h_inf, l, l_inf, precompute=False, vk_inf=None):
         """vk_inf: optional is_infinity flags of (delta_g1, alpha_g1, beta_g1).  An identity delta_g1 raises ProverSubVersionCrsAttack
         before anything is uploaded — the reference returns that error from create_proof (prover.rs:67-69)."""
+        self._set_vk(delta_g1, alpha_g1, beta_g1, vk_inf)
+        self._set_queries(*(Bases(BN254_G1, p, f) for p, f in ((a, a_inf), (b_g1, b_g1_inf), (h, h_inf), (l, l_inf))), precompute=precompute)
+
+    @classmethod
+    def from_params(cls, params, precompute=False):
+        """A prover on the resident queries of `params` (groth16.setup): no download, no re-upload.  The prover takes the handles over
+        (Groth16Params.take) and frees them once, in `free`."""
+        self = cls.__new__(cls)
+        self._adopt(params, precompute)
+        return self
+
+    def _adopt(self, params, precompute):
+        alpha, beta, delta = params.vk_g1
+        self._set_vk(delta[:8], alpha[:8], beta[:8], [delta[8], alpha[8], beta[8]])
+        self._set_queries(*params.take("a", "b_g1", "h", "l"), precompute=precompute)
+
+    def _set_vk(self, delta_g1, alpha_g1, beta_g1, vk_inf):
         self.vk, self.vk_inf = _vk_points([delta_g1, alpha_g1, beta_g1], vk_inf, 8)
         if self.vk_inf[0]:
             raise ProverSubVersionCrsAttack("vk.delta_g1 is the identity")
-        self.a, self.b_g1, self.h, self.l = (Bases(BN254_G1, p, f) for p, f in ((a, a_inf), (b_g1, b_g1_inf), (h, h_inf), (l, l_inf)))
+
+    def _set_queries(self, a, b_g1, h, l, precompute):
+        self.a, self.b_g1, self.h, self.l = a, b_g1, h, l
         self.vk_bases = Bases(BN254_G1, self.vk, self.vk_inf)
         if precompute:
             for b in (self.a, self.b_g1, self.h, self.l):
@@ -119,11 +206,25 @@ class Groth16Prover(Groth16G1Prover):
     def __init__(self, delta_g1, alpha_g1, beta_g1, a, a_inf, b_g1, b_g1_inf, h, h_inf, l, l_inf, delta_g2, beta_g2, b_g2, b_g2_inf, precompute=False,
                  vk_inf=None, vk_g2_inf=None):
         """vk_g2_inf: optional is_infinity flags of (delta_g2, beta_g2); an identity delta_g2 raises ProverSubVersionCrsAttack (prover.rs:67-69)."""
+        self._set_vk_g2(delta_g2, beta_g2, vk_g2_inf)
+        super().__init__(delta_g1, alpha_g1, beta_g1, a, a_inf, b_g1, b_g1_inf, h, h_inf, l, l_inf, precompute=precompute, vk_inf=vk_inf)
+        self._set_g2_query(Bases(BN254_G2, b_g2, b_g2_inf), precompute)
+
+    def _adopt(self, params, precompute):
+        if params.b_g2 is None:
+            raise ValueError("the parameters hold no b_g2 query (setup with g2=False, or already taken)")
+        beta, _, delta = params.vk_g2
+        self._set_vk_g2(delta[:16], beta[:16], [delta[16], beta[16]])
+        super()._adopt(params, precompute)
+        self._set_g2_query(*params.take("b_g2"), precompute)
+
+    def _set_vk_g2(self, delta_g2, beta_g2, vk_g2_inf):
         self.vk_g2, self.vk_g2_inf = _vk_points([delta_g2, beta_g2], vk_g2_inf, 16)
         if self.vk_g2_inf[0]:
             raise ProverSubVersionCrsAttack("vk.delta_g2 is the identity")
-        super().__init__(delta_g1, alpha_g1, beta_g1, a, a_inf, b_g1, b_g1_inf, h, h_inf, l, l_inf, precompute=precompute, vk_inf=vk_inf)
-        self.b_g2 = Bases(BN254_G2, b_g2, b_g2_inf)
+
+    def _set_g2_query(self, b_g2, precompute):
+        self.b_g2 = b_g2
         self.vk_g2_bases = Bases(BN254_G2, self.vk_g2, self.vk_g2_inf)
         if precompute:
             self.b_g2.precompute(0)

@@ -178,6 +178,34 @@ def groth16_prove_r1cs(log_n, shape, z, n_inputs, h, l, a, b_g1, b_g2, jobs, wan
     return res, (q[: q_len.value] if want_q else None), outs
 
 
+SETUP_QUERIES = ("h", "l", "a", "b_g1", "b_g2", "ic")
+
+
+def groth16_setup(shape, n_inputs, toxic, g2=True):
+    """kgr_groth16_setup: groth16/src/zksnark.rs:17-127 on the device from a registered R1CS shape (nova.R1csShape over Fr).  toxic: (5, 4) uint64
+    Montgomery alpha, beta, gamma, delta, tau.  -> (log_n, {query name: Bases} (no "b_g2" without g2), vk_g1 (3, 9), vk_g2 (3, 17) or None)."""
+    _lib.ensure_init()
+    toxic = _c(toxic).reshape(5, 4)
+    handles = [ctypes.c_void_p() for _ in SETUP_QUERIES]
+    log_n = ctypes.c_uint32()
+    vk_g1 = np.zeros((3, 9), dtype=np.uint64)
+    vk_g2 = np.zeros((3, 17), dtype=np.uint64) if g2 else None
+    refs = [ctypes.byref(h) if name != "b_g2" or g2 else None for name, h in zip(SETUP_QUERIES, handles)]
+    _lib.check(_lib.lib().kgr_groth16_setup(shape._h, n_inputs, _u64(toxic), ctypes.byref(log_n), *refs, _u64(vk_g1), _u64(vk_g2) if g2 else None))
+    L = _lib.lib()
+    queries = {name: Bases(BN254_G2 if name == "b_g2" else BN254_G1, _handle=h, _n=L.kgr_bases_len(h))
+               for name, h in zip(SETUP_QUERIES, handles) if name != "b_g2" or g2}
+    return int(log_n.value), queries, vk_g1, vk_g2
+
+
+def groth16_setup_timing():
+    """Device time (ms) per phase of the last groth16_setup (kgr_groth16_setup_last_timing)."""
+    ms = (ctypes.c_float * 10)()
+    _lib.check(_lib.lib().kgr_groth16_setup_last_timing(ms))
+    keys = ["powers_idft", "columns", "scalars", "a", "b_g1", "ic", "l", "h", "b_g2", "vk"]
+    return dict(zip(keys, [float(x) for x in ms]))
+
+
 def msm_device(bases, d_scalars_ptr, n, scalar_fmt=SCALARS_MONTGOMERY, base_off=0):
     """MSM with the scalars already in device memory (raw pointer, n x 4 uint64)."""
     out = np.zeros(3 * coord_limbs(bases.curve), dtype=np.uint64)

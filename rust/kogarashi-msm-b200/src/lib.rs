@@ -82,6 +82,10 @@ extern "C" {
     fn kgr_groth16_prove_r1cs(log_n: u32, cs: *const kgr_r1cs_t, z: *const kgr_vec_t, n_inputs: usize, h: *mut kgr_bases_t, l: *mut kgr_bases_t,
                               a: *mut kgr_bases_t, b_g1: *mut kgr_bases_t, b_g2: *mut kgr_bases_t, out: *mut u64, q_out: *mut u64, q_len: *mut usize,
                               jobs: *const kgr_msm_job_t, n_jobs: usize) -> i32;
+    fn kgr_groth16_setup(cs: *const kgr_r1cs_t, n_inputs: usize, toxic: *const u64, log_n_out: *mut u32, h: *mut *mut kgr_bases_t,
+                         l: *mut *mut kgr_bases_t, a: *mut *mut kgr_bases_t, b_g1: *mut *mut kgr_bases_t, b_g2: *mut *mut kgr_bases_t,
+                         ic: *mut *mut kgr_bases_t, vk_g1: *mut u64, vk_g2: *mut u64) -> i32;
+    fn kgr_groth16_setup_last_timing(ms: *mut f32) -> i32;
     fn kgr_set_param(name: *const c_char, value: c_long) -> i32;
     fn kgr_last_timing(dev: i32, ms: *mut f32, shape: *mut u32) -> i32;
     fn kgr_event_record(dev: i32, idx: i32) -> i32;
@@ -392,6 +396,42 @@ impl GpuProver {
         ProverQueries { q: G1Affine::extended_from_limbs(&out[0..12]), l: G1Affine::extended_from_limbs(&out[12..24]),
                         a_answer: G1Affine::extended_from_limbs(&out[24..36]), b1_answer: G1Affine::extended_from_limbs(&out[36..48]),
                         b2_answer: G2Affine::extended_from_limbs(&out[48..72]) }
+    }
+}
+
+/// `Parameters` of `ZkSnark::setup` (groth16/src/zksnark.rs:17-127) generated on the GPU by `kgr_groth16_setup` (uncompiled, like the rest of this
+/// file): the queries stay resident, the verifying key comes back as limbs (`vk_g1`: alpha, beta, delta as x[4] y[4] is_infinity; `vk_g2`: beta,
+/// gamma, delta as x[8] y[8] is_infinity).  The h query has m - 1 entries as the reference's: proofs are guaranteed valid for m = 2^log_n only.
+pub struct GpuParams {
+    pub log_n: u32,
+    pub prover: GpuProver,
+    pub ic: RegisteredBases<bn_254::G1Affine>,
+    pub vk_g1: [u64; 27],
+    pub vk_g2: [u64; 51],
+}
+
+impl GpuParams {
+    /// `cs`: the circuit's shape over Fr (columns `Wire::Instance(i) -> i`, `Wire::Witness(i) -> n_inputs + i`); `toxic`: alpha, beta, gamma, delta,
+    /// tau (the five `Fr::random` draws of zksnark.rs:24-28).  The b_g2 query is always built here (the prover needs it).
+    pub fn setup(cs: &R1csShapeGpu, n_inputs: usize, toxic: [bn_254::Fr; 5]) -> Self {
+        let tox: Vec<u64> = toxic.iter().flat_map(|t| t.0).collect();
+        let mut log_n = 0u32;
+        let mut hs = [core::ptr::null_mut(); 6];
+        let (mut vk_g1, mut vk_g2) = ([0u64; 27], [0u64; 51]);
+        let [h, l, a, b_g1, b_g2, ic] = &mut hs;
+        check(unsafe { kgr_groth16_setup(cs.handle, n_inputs, tox.as_ptr(), &mut log_n, h, l, a, b_g1, b_g2, ic, vk_g1.as_mut_ptr(), vk_g2.as_mut_ptr()) });
+        fn adopt<C: GpuCurve>(handle: *mut kgr_bases_t) -> RegisteredBases<C> {
+            RegisteredBases { handle, len: unsafe { kgr_bases_len(handle) }, _curve: core::marker::PhantomData }
+        }
+        let prover = GpuProver { h: adopt(hs[0]), l: adopt(hs[1]), a: adopt(hs[2]), b_g1: adopt(hs[3]), b_g2: adopt(hs[4]) };
+        Self { log_n, prover, ic: adopt(hs[5]), vk_g1, vk_g2 }
+    }
+
+    /// Device time (ms) of the phases of the last setup (`kgr_groth16_setup_last_timing`).
+    pub fn last_timing() -> [f32; 10] {
+        let mut ms = [0f32; 10];
+        check(unsafe { kgr_groth16_setup_last_timing(ms.as_mut_ptr()) });
+        ms
     }
 }
 

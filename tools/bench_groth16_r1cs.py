@@ -5,6 +5,7 @@ circuit (the example's x^3 + x + 5 iterated) at 2^16 and 2^20 constraints.  One 
   z_upload_ms                best-of-N wall time of the DeviceVec upload of z (what a caller with z in host memory adds to prove_r1cs)
   host_evaluate_s            cs.evaluate() as the old path needs it: the C++ oracle's SparseMatrix::prod (zkstd/src/matrix.rs:36-48) x 3, one core
   same_proof                 A, B, C and q of the two paths byte for byte, and the oracle's evaluations equal the host ones
+  device_crs_setup_s         wall time of groth16.setup, which generates the CRS both provers use on the device
   h2d_bytes_per_call         per path, from the shapes
 usage: python tools/bench_groth16_r1cs.py --out DIR [--logm 16 20] [--steps 5] [--warmup 3]"""
 import argparse
@@ -14,15 +15,12 @@ import subprocess
 import sys
 import time
 
-import numpy as np
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import kogarashi_b200 as k  # noqa: E402
 from groth16_r1cs_util import csr_from_r1cs, mont  # noqa: E402
-from kogarashi_b200 import msm as M  # noqa: E402
-from kogarashi_b200.groth16 import Groth16Prover  # noqa: E402
+from kogarashi_b200.groth16 import Groth16Prover, setup  # noqa: E402
 from kogarashi_b200.nova import FIELD_FR, DeviceVec, R1csShape  # noqa: E402
 from oracle import groth16_ref as G  # noqa: E402
 from oracle import oracle as A  # noqa: E402
@@ -48,24 +46,21 @@ def card():
 def bench(logm, steps, warmup):
     t0 = time.perf_counter()
     cs, _ = G.chain_circuit(((1 << logm) - 1) // 3, 3)
-    E, trap, uvw = G.crs_exponents(cs, B.XorShift128(A.DEFAULT_SEED))
     m, n_z, mats = csr_from_r1cs(cs)
     evals = tuple(mont(v) for v in cs.evaluate())
     z, xs, ws = mont(cs.x + cs.w), mont(cs.x), mont(cs.w)
     setup_s = time.perf_counter() - t0
-
-    def points(curve, exps):
-        return M.fixed_base_mul(curve, mont(exps)), np.array([1 if e == 0 else 0 for e in exps], dtype=np.uint8)
-
-    vk = points(k.BN254_G1, [trap["delta"], trap["alpha"], trap["beta"]])[0]
-    vk2 = points(k.BN254_G2, [trap["delta"], trap["beta"]])[0]
-    crs = [points(k.BN254_G1, E[name]) for name in ("a", "b_g1", "h", "l")]
-    prover = Groth16Prover(vk[0], vk[1], vk[2], *crs[0], *crs[1], *crs[2], *crs[3], vk2[0], vk2[1], *points(k.BN254_G2, E["b_g1"]))
+    shape, zv = R1csShape(FIELD_FR, m, n_z, *mats), DeviceVec(FIELD_FR, z)
+    rng = B.XorShift128(A.DEFAULT_SEED)
+    t0 = time.perf_counter()
+    params = setup(shape, cs.l, toxic=[rng.random_field(B.FR) for _ in range(5)])   # the CRS on the device (zksnark.rs:17-127)
+    crs_s = time.perf_counter() - t0
+    log_n = params.log_n
+    prover = Groth16Prover.from_params(params)
     rng = B.XorShift128(bytes(range(1, 17)))
     r, s = rng.random_field(B.FR), rng.random_field(B.FR)
-    shape, zv = R1csShape(FIELD_FR, m, n_z, *mats), DeviceVec(FIELD_FR, z)
-    old = lambda: prover.prove_from_evaluations(E["k"], *evals, xs, ws, r, s)
-    new = lambda: prover.prove_r1cs(E["k"], shape, zv, cs.l, r, s)
+    old = lambda: prover.prove_from_evaluations(log_n, *evals, xs, ws, r, s)
+    new = lambda: prover.prove_r1cs(log_n, shape, zv, cs.l, r, s)
     for _ in range(warmup):
         old(), new()
     t_old, t_new = [], []
@@ -88,7 +83,7 @@ def bench(logm, steps, warmup):
     blind = (2 + 2) * el   # the two blinding jobs of Groth16Prover: [r, 1] and [s, 1]
     rec = {
         "workload": "Groth16 create_proof of the chain circuit (x^3 + x + 5 iterated) after synthesis: prover.rs:32-98",
-        "constraints": m, "n_z": n_z, "log_n": E["k"], "steps": steps, "warmup": warmup,
+        "constraints": m, "n_z": n_z, "log_n": log_n, "steps": steps, "warmup": warmup,
         "prove_from_evaluations_ms": min(t_old) * 1e3, "prove_r1cs_ms": min(t_new) * 1e3, "z_upload_ms": min(t_up) * 1e3,
         "host_evaluate_s": min(t_eval), "host_evaluate_cores": 1,
         "host_evaluate_note": "C++ oracle SparseMatrix::prod x 3 (A z, B z, C z), a serial loop on one core; the Python restatement is not timed",
@@ -96,9 +91,9 @@ def bench(logm, steps, warmup):
         "h2d_bytes_per_call": {"prove_from_evaluations": 3 * m * el + 3 * n_z * el + (n_z - l) * el + blind, "prove_r1cs": blind,
                                "z_upload_if_z_is_on_the_host": n_z * el,
                                "note": "old: a, b, c + z for the a, b_g1, b_g2 lanes + aux for l + blinding scalars; new: blinding scalars only"},
-        "python_setup_s": setup_s, "card": card(),
+        "python_setup_s": setup_s, "device_crs_setup_s": crs_s, "card": card(),
     }
-    shape.free(), zv.free(), prover.free()
+    shape.free(), zv.free(), prover.free(), params.free()
     return rec
 
 
