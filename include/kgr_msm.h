@@ -220,6 +220,28 @@ int kgr_groth16_setup(const kgr_r1cs_t *cs, size_t n_inputs, const uint64_t toxi
  * of a device are built before [0] and are not included. */
 int kgr_groth16_setup_last_timing(float ms[10]);
 
+/* Reduced optimal-ate pairing on BN254 (the map the Groth16 check of groth16/src/proof.rs:39-48 evaluates).
+ * g1: n x 9 words (x[4] y[4] is_infinity, Montgomery Fq), g2: n x 17 (x.c0 x.c1 y.c0 y.c1 is_infinity); a set flag means the identity.
+ * op 0: out = n x 48 words, e(P_i, Q_i) each;  op 1: out = 48 words, prod_i e(P_i, Q_i) (one final exponentiation; n == 0 gives 1).
+ * Gt is 12 Fq elements, Montgomery, order c0.c0.c0, c0.c0.c1, c0.c1.c0, ..., c1.c2.c1 (Fq12 = c0 + c1 w, Fq6 = c0 + c1 v + c2 v^2,
+ * w^2 = v, v^3 = 9 + u).  A pair with an identity contributes 1.
+ * Points off their curve, a G2 point outside G2, or a coordinate >= p: KGR_E_ARG. */
+int kgr_pairing(const uint64_t *g1, const uint64_t *g2, size_t n, int op, uint64_t *out);
+
+/* Groth16 verification of k proofs against one verifying key (groth16/src/verifier.rs).  vk_g1: alpha, beta, delta (3 x 9), vk_g2: beta,
+ * gamma, delta (3 x 17), the layout kgr_groth16_setup writes; ic: a BN254 G1 handle of n_public + 1 points (ic_0 carries the constant one).
+ * proofs: k x 35 = A[9] B[17] C[9], the prover's output.  inputs: k x n_public x 4 Montgomery Fr, the instance WITHOUT its leading one.
+ * ok[i] = 1 iff  e(A_i, B_i) = e(alpha, beta) e(ic_0 + sum_j x_ij ic_{j+1}, gamma) e(C_i, delta)  and every point of proof i is valid (each
+ * coordinate < p, A and C on the curve, B on the twist and in G2; a set is_infinity flag is the identity).  A failing proof gets 0, not an error.
+ * k >= 2 needs rho (k x 2 words, 128-bit, non-zero, unpredictable to whoever made the proofs): one batched check
+ *   prod_i e(rho_i A_i, B_i) * e(-sum_i rho_i IC(x_i), gamma) * e(-sum_i rho_i C_i, delta) * e(-(sum_i rho_i) alpha, beta) == 1
+ * over the valid proofs; if it fails, every proof is checked on its own.  k == 1: the per-proof check (rho ignored).
+ * KGR_E_ARG before any work: NULL pointers, ic not a single-shard G1 handle of the current kgr_init, n_public + 1 != ic->n, an input >= r,
+ * k >= 2 without rho or with a zero rho_i, an invalid verifying-key point, an identity gamma or delta, a context of more than one device.
+ * k == 0: KGR_OK, nothing done. */
+int kgr_groth16_verify(const uint64_t *vk_g1, const uint64_t *vk_g2, kgr_bases_t *ic, const uint64_t *proofs, size_t k,
+                       const uint64_t *inputs, size_t n_public, const uint64_t *rho, uint32_t *ok);
+
 /* Tuning knobs: "window_bits" (0 = auto), "chunk" (entries per accumulate thread, 0 = auto),
  * "reduce_fanin" (power of two), "running_sum_stop" (elements per window below which the reduce
  * switches from running sums to the parallel weighting pass), "final_on_device" (1: Horner over

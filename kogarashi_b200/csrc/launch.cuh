@@ -124,4 +124,31 @@ struct LaunchSetup {
                        void *ext, void *h);
 };
 
+// BN254 pairing and Groth16 verification (kernels_pairing.cu, bodies in pairing.cuh).  Points are device affine forms (G1 64 bytes, G2 128
+// bytes, the identity (0, 0)), Fq12 values 384 bytes, lines 192 bytes (MILLER_LINES per fixed G2 point), XYZZ G1 points 128 bytes.
+struct LaunchPairing {
+    static constexpr size_t G1_BYTES = 64, G2_BYTES = 128, FQ12_BYTES = 384, LINE_BYTES = 192, XYZZ_BYTES = 128;
+    // ABI rows (9 / 17 words) -> device points; *bad |= 1 if any point is invalid
+    static void load(cudaStream_t st, uint32_t n, const uint64_t *g1, const uint64_t *g2, void *p, void *q, uint32_t *bad);
+    // proofs: k x 35 words; valid: k bytes; inputs_canon: k x n_public canonical Fr (32 bytes)
+    static void validate_proofs(cudaStream_t st, uint32_t k, const uint64_t *proofs, const uint64_t *inputs, uint32_t n_public, void *a, void *b, void *c,
+                                uint8_t *valid, void *inputs_canon);
+    static void lines(cudaStream_t st, uint32_t n, const void *q, void *table);
+    static void miller(cudaStream_t st, uint32_t n, const void *p, const void *q, void *f);
+    // ceil(log2 n) levels ping-ponging between f[0] and f[1] (and sums[0] / sums[1], 2 XYZZ points per element, unless sums == nullptr); the
+    // product lands in element 0 of buffer `root`.  Returns the launches.
+    static int product_tree(cudaStream_t st, uint32_t n, void *f[2], void *sums[2], int &root);
+    static int tree_levels(uint32_t n);
+    static void final_exp(cudaStream_t st, uint32_t n, const void *f, void *out_gt, const uint8_t *valid, uint32_t *ok);
+    // rho: k x 2 words; sums: 2 XYZZ points per proof (rho_i C_i, rho_i alpha); rho_mont: k x 32 bytes
+    static void batch_prep(cudaStream_t st, uint32_t k, const uint64_t *rho, const uint8_t *valid, const void *a, const void *c, const void *alpha,
+                           void *rho_a, void *sums, void *rho_mont);
+    static void batch_colsum(cudaStream_t st, uint32_t k, uint32_t n_public, const void *rho_mont, const uint64_t *inputs, void *out);
+    static void batch_fixed(cudaStream_t st, const void *f_root, const void *sums_root, const void *ic_sum, const void *lines, uint32_t present, void *out);
+    static void ic_table(cudaStream_t st, uint32_t n_public, const void *ic, void *table);
+    static void ic_straus(cudaStream_t st, uint32_t k, uint32_t n_public, const void *ic, const void *table, const void *inputs_canon, void *ic_x);
+    static void verify_miller(cudaStream_t st, uint32_t k, const void *a, const void *b, const void *c, const void *alpha, const void *ic_x,
+                              const void *lines, uint32_t present, void *f);
+};
+
 }  // namespace kgr

@@ -34,6 +34,7 @@
 
 #include "../../include/kgr_msm.h"
 #include "launch.cuh"
+#include "pairing.cuh"
 #include "r1cs_kernels.cuh"
 #include "setup_kernels.cuh"
 
@@ -2630,6 +2631,167 @@ int kgr_groth16_setup_last_timing(float ms[10]) {
     if (!ms) return fail(KGR_E_ARG, "null pointer");
     std::memcpy(ms, g_setup_ms, sizeof g_setup_ms);
     return KGR_OK;
+}
+
+// ---- BN254 pairing and Groth16 verification (groth16/src/verifier.rs: the check of proof.rs:39-48) on the device --------------------------
+int kgr_pairing(const uint64_t *g1, const uint64_t *g2, size_t n, int op, uint64_t *out) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (g_engines.empty()) return fail(KGR_E_NOT_INIT, "kgr_init has not been called");
+    if (!out || (n && (!g1 || !g2))) return fail(KGR_E_ARG, "null pointer");
+    if (op != 0 && op != 1) return fail(KGR_E_ARG, "op must be 0 (one value per pair) or 1 (the product)");
+    if (n >= (1ull << 31)) return fail(KGR_E_TOO_LARGE, "at most 2^31 - 1 pairs");
+    if (n == 0) {
+        if (op == 1) {
+            const Fq12 one = fq12_one();
+            std::memcpy(out, &one, sizeof one);
+        }
+        return KGR_OK;
+    }
+    return guarded([&]() -> int {
+        Engine &e = g_engines[0];
+        CK(cudaSetDevice(e.dev));
+        struct Scratch {
+            DevBuf<uint64_t> g1, g2;
+            DevBuf<uint8_t> p, q, f[2], gt;
+            DevBuf<uint32_t> bad;
+            ~Scratch() {
+                g1.release(), g2.release(), bad.release();
+                for (auto *b : {&p, &q, &f[0], &f[1], &gt}) b->release();
+            }
+        } sc;
+        typedef LaunchPairing L;
+        sc.g1.ensure(9 * n), sc.g2.ensure(17 * n), sc.p.ensure(n * L::G1_BYTES), sc.q.ensure(n * L::G2_BYTES), sc.bad.ensure(1);
+        sc.f[0].ensure(n * L::FQ12_BYTES), sc.f[1].ensure(((n + 1) / 2) * L::FQ12_BYTES), sc.gt.ensure((op ? 1 : n) * L::FQ12_BYTES);
+        CK(cudaMemcpyAsync(sc.g1.p, g1, 72 * n, cudaMemcpyHostToDevice, e.st));
+        CK(cudaMemcpyAsync(sc.g2.p, g2, 136 * n, cudaMemcpyHostToDevice, e.st));
+        CK(cudaMemsetAsync(sc.bad.p, 0, 4, e.st));
+        L::load(e.st, (uint32_t)n, sc.g1.p, sc.g2.p, sc.p.p, sc.q.p, sc.bad.p);
+        L::miller(e.st, (uint32_t)n, sc.p.p, sc.q.p, sc.f[0].p);
+        e.launches += 2;
+        int root = 0;
+        void *fb[2] = {sc.f[0].p, sc.f[1].p};
+        if (op == 1) e.launches += L::product_tree(e.st, (uint32_t)n, fb, nullptr, root);
+        L::final_exp(e.st, op ? 1u : (uint32_t)n, sc.f[root].p, sc.gt.p, nullptr, nullptr);
+        e.launches++;
+        CK(cudaGetLastError());
+        uint32_t bad = 0;
+        CK(cudaMemcpyAsync(&bad, sc.bad.p, 4, cudaMemcpyDeviceToHost, e.st));
+        CK(cudaStreamSynchronize(e.st));
+        if (bad) return fail(KGR_E_ARG, "a G1 point off the curve, a G2 point off the twist or outside G2, or a coordinate >= p");
+        CK(cudaMemcpyAsync(out, sc.gt.p, (op ? 1 : n) * L::FQ12_BYTES, cudaMemcpyDeviceToHost, e.st));
+        CK(cudaStreamSynchronize(e.st));
+        return KGR_OK;
+    });
+}
+
+int kgr_groth16_verify(const uint64_t *vk_g1, const uint64_t *vk_g2, kgr_bases_t *ic, const uint64_t *proofs, size_t k, const uint64_t *inputs,
+                       size_t n_public, const uint64_t *rho, uint32_t *ok) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (g_engines.empty()) return fail(KGR_E_NOT_INIT, "kgr_init has not been called");
+    if (!vk_g1 || !vk_g2 || !ic || (k && (!proofs || !ok || (n_public && !inputs)))) return fail(KGR_E_ARG, "null pointer");
+    if (int rc = query_check(ic, KGR_CURVE_BN254_G1, "ic")) return rc;
+    if (n_public + 1 != ic->n) return fail(KGR_E_ARG, "ic must hold n_public + 1 points (ic_0 carries the constant one)");
+    if (g_engines.size() != 1) return fail(KGR_E_ARG, "verification needs a single-device context");
+    if (k >= (1ull << 31) || (k && n_public >= (1ull << 31) / k)) return fail(KGR_E_TOO_LARGE, "too many proofs or inputs");
+    if (k >= 2) {
+        if (!rho) return fail(KGR_E_ARG, "a batch of two or more proofs needs rho");
+        for (size_t i = 0; i < k; i++)
+            if (!(rho[2 * i] | rho[2 * i + 1])) return fail(KGR_E_ARG, "every rho_i must be non-zero");
+    }
+    for (size_t i = 0; i < k * n_public; i++)
+        if (!fr_canonical(inputs + 4 * i)) return fail(KGR_E_ARG, "public inputs must be reduced modulo r");
+    G1A vk1[3];
+    G2A vk2[3];
+    for (int j = 0; j < 3; j++)
+        if (!load_g1(vk_g1 + 9 * j, vk1[j])) return fail(KGR_E_ARG, "a G1 point of the verifying key is invalid");
+    uint32_t present = 0;
+    for (int j = 0; j < 3; j++) {
+        if (!load_g2(vk_g2 + 17 * j, vk2[j])) return fail(KGR_E_ARG, "a G2 point of the verifying key is invalid (off the twist or outside G2)");
+        if (!affine_is_identity(vk2[j])) present |= 1u << j;
+    }
+    if ((present & 6u) != 6u) return fail(KGR_E_ARG, "gamma and delta must not be the identity");
+    if (k == 0) return KGR_OK;
+    return guarded([&]() -> int {
+        typedef LaunchPairing L;
+        Engine &e = g_engines[0];
+        CK(cudaSetDevice(e.dev));
+        const uint32_t K = (uint32_t)k, NP = (uint32_t)n_public;
+        struct Scratch {
+            DevBuf<uint64_t> proofs, inputs, rho;
+            DevBuf<uint8_t> a, b, c, valid, canon, fixed, lines, f[2], sums[2], rho_a, rho_mont, colsum, fbatch, ic_tab, ic_x;
+            DevBuf<uint32_t> ok;
+            ~Scratch() {
+                proofs.release(), inputs.release(), rho.release(), ok.release();
+                for (auto *x : {&a, &b, &c, &valid, &canon, &fixed, &lines, &f[0], &f[1], &sums[0], &sums[1], &rho_a, &rho_mont, &colsum, &fbatch, &ic_tab,
+                                &ic_x})
+                    x->release();
+            }
+        } sc;
+        sc.proofs.ensure(35 * k), sc.inputs.ensure(std::max<size_t>(4 * k * n_public, 1));
+        sc.a.ensure(k * L::G1_BYTES), sc.b.ensure(k * L::G2_BYTES), sc.c.ensure(k * L::G1_BYTES), sc.valid.ensure(k);
+        sc.canon.ensure(std::max<size_t>(k * n_public, 1) * 32), sc.lines.ensure(3 * MILLER_LINES * L::LINE_BYTES);
+        sc.fixed.ensure(2 * L::G1_BYTES + 3 * L::G2_BYTES);  // alpha, the batched IC sum, beta, gamma, delta
+        sc.f[0].ensure(k * L::FQ12_BYTES), sc.f[1].ensure(((k + 1) / 2) * L::FQ12_BYTES), sc.ok.ensure(k + 1);
+        uint8_t *d_alpha = sc.fixed.p, *d_icsum = sc.fixed.p + L::G1_BYTES, *d_vk2 = sc.fixed.p + 2 * L::G1_BYTES;
+        CK(cudaMemcpyAsync(sc.proofs.p, proofs, 35 * 8 * k, cudaMemcpyHostToDevice, e.st));
+        if (n_public) CK(cudaMemcpyAsync(sc.inputs.p, inputs, 32 * k * n_public, cudaMemcpyHostToDevice, e.st));
+        CK(cudaMemcpyAsync(d_alpha, &vk1[0], sizeof(G1A), cudaMemcpyHostToDevice, e.st));
+        CK(cudaMemcpyAsync(d_vk2, vk2, sizeof vk2, cudaMemcpyHostToDevice, e.st));
+        L::validate_proofs(e.st, K, sc.proofs.p, sc.inputs.p, NP, sc.a.p, sc.b.p, sc.c.p, sc.valid.p, sc.canon.p);
+        L::lines(e.st, 3, d_vk2, sc.lines.p);
+        e.launches += 2;
+        CK(cudaGetLastError());
+        std::vector<uint8_t> valid(k);
+        if (k >= 2) {
+            // one random linear combination of the k checks: a single final exponentiation
+            sc.rho.ensure(2 * k), sc.rho_a.ensure(k * L::G1_BYTES), sc.rho_mont.ensure(k * 32), sc.colsum.ensure((n_public + 1) * 32);
+            sc.sums[0].ensure(2 * k * L::XYZZ_BYTES), sc.sums[1].ensure(2 * ((k + 1) / 2) * L::XYZZ_BYTES), sc.fbatch.ensure(L::FQ12_BYTES);
+            CK(cudaMemcpyAsync(sc.rho.p, rho, 16 * k, cudaMemcpyHostToDevice, e.st));
+            L::batch_prep(e.st, K, sc.rho.p, sc.valid.p, sc.a.p, sc.c.p, d_alpha, sc.rho_a.p, sc.sums[0].p, sc.rho_mont.p);
+            L::batch_colsum(e.st, K, NP, sc.rho_mont.p, sc.inputs.p, sc.colsum.p);
+            e.launches += 2;
+            CK(cudaGetLastError());
+            // sum_i rho_i IC(x_i) = (sum_i rho_i) ic_0 + sum_j s_j ic_{j+1}: one MSM over the ic handle with device-resident scalars
+            uint64_t proj[12], aff[9];
+            run_msm<Bn254G1>(ic->shards, 0, reinterpret_cast<const uint64_t *>(sc.colsum.p), true, KGR_SCALARS_MONTGOMERY, n_public + 1, proj, nullptr);
+            proj_to_affine_host<Bn254G1>(proj, aff);
+            G1A icsum{};
+            if (!aff[8]) std::memcpy(&icsum, aff, sizeof icsum);
+            CK(cudaMemcpyAsync(d_icsum, &icsum, sizeof icsum, cudaMemcpyHostToDevice, e.st));
+            L::miller(e.st, K, sc.rho_a.p, sc.b.p, sc.f[0].p);
+            e.launches++;
+            int root = 0;
+            void *fb[2] = {sc.f[0].p, sc.f[1].p}, *sb[2] = {sc.sums[0].p, sc.sums[1].p};
+            e.launches += L::product_tree(e.st, K, fb, sb, root);
+            L::batch_fixed(e.st, sc.f[root].p, sc.sums[root].p, d_icsum, sc.lines.p, present, sc.fbatch.p);
+            L::final_exp(e.st, 1, sc.fbatch.p, nullptr, nullptr, sc.ok.p + k);
+            e.launches += 2;
+            CK(cudaGetLastError());
+            uint32_t batch_ok = 0;
+            CK(cudaMemcpyAsync(&batch_ok, sc.ok.p + k, 4, cudaMemcpyDeviceToHost, e.st));
+            CK(cudaMemcpyAsync(valid.data(), sc.valid.p, k, cudaMemcpyDeviceToHost, e.st));
+            CK(cudaStreamSynchronize(e.st));
+            if (batch_ok) {
+                for (size_t i = 0; i < k; i++) ok[i] = valid[i];
+                return KGR_OK;
+            }
+        }
+        // every proof on its own: IC(x_i) by Straus over the ic points, one multi-Miller loop and one final exponentiation per thread
+        const void *ic_pts = ic->shards[0].d_pts;
+        sc.ic_tab.ensure(std::max<size_t>(16 * n_public, 1) * L::G1_BYTES), sc.ic_x.ensure(k * L::G1_BYTES);
+        if (NP) {
+            L::ic_table(e.st, NP, ic_pts, sc.ic_tab.p);
+            e.launches++;
+        }
+        L::ic_straus(e.st, K, NP, ic_pts, sc.ic_tab.p, sc.canon.p, sc.ic_x.p);
+        L::verify_miller(e.st, K, sc.a.p, sc.b.p, sc.c.p, d_alpha, sc.ic_x.p, sc.lines.p, present, sc.f[0].p);
+        L::final_exp(e.st, K, sc.f[0].p, nullptr, sc.valid.p, sc.ok.p);
+        e.launches += 3;
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(ok, sc.ok.p, 4 * k, cudaMemcpyDeviceToHost, e.st));
+        CK(cudaStreamSynchronize(e.st));
+        return KGR_OK;
+    });
 }
 
 int kgr_host_alloc(size_t bytes, void **out) {

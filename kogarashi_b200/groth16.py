@@ -14,6 +14,8 @@ of its slice layout, :58-62).  The blinding terms are a five-point MSM, so no cu
 R1CS shape and the resident assignment z, and every query reads its scalars from z in device memory.
 `setup` generates the parameters themselves (groth16/src/zksnark.rs:17-127) on the device from the registered shape; `from_params` hands its
 resident queries to a prover without a download or a re-upload.
+`Groth16Verifier` checks proofs (groth16/src/verifier.rs, the pairing equation of proof.rs:39-48) on the device, one batched pairing check for
+a set of proofs against one key.
 """
 import os
 
@@ -21,7 +23,7 @@ import numpy as np
 
 from .fft import Fft
 from .msm import (BN254_G1, BN254_G2, SCALARS_CANONICAL, SCALARS_MONTGOMERY, Bases, coord_limbs, groth16_msms, groth16_prove_r1cs, groth16_setup,
-                  msm_batch, msm_curve_addition, proj_add, to_affine)
+                  groth16_verify, msm_batch, msm_curve_addition, proj_add, to_affine)
 
 FR = 0x30644E72E131A029B85045B68181585D2833E84879B9709143E1F593F0000001  # bn254/src/fr.rs:11-16
 
@@ -270,3 +272,56 @@ class Groth16Prover(Groth16G1Prover):
         super().free()
         self.b_g2.free()
         self.vk_g2_bases.free()
+
+
+class Groth16Verifier:
+    """groth16/src/verifier.rs on the device (kgr_groth16_verify).  vk_g1 (3, 9): alpha, beta, delta; vk_g2 (3, 17): beta, gamma, delta (the layout
+    of Groth16Params); ic: the ic query as `Bases`, or a host (points (n, 8), is_infinity (n,)) pair that is registered here and freed in `free`."""
+
+    def __init__(self, vk_g1, vk_g2, ic):
+        self.vk_g1 = np.ascontiguousarray(vk_g1, dtype=np.uint64).reshape(3, 9)
+        self.vk_g2 = np.ascontiguousarray(vk_g2, dtype=np.uint64).reshape(3, 17)
+        if isinstance(ic, Bases):
+            self.ic, self._own_ic = ic, False
+        else:
+            pts, inf = ic
+            self.ic, self._own_ic = Bases(BN254_G1, pts, inf), True
+
+    @classmethod
+    def from_params(cls, params):
+        """A verifier on the resident ic query of `params` (groth16.setup): borrowed, not taken, so the parameters keep it and free it."""
+        if params.ic is None or params.vk_g2 is None:
+            raise ValueError("the parameters hold no ic query or no G2 verifying key (setup with g2=False)")
+        return cls(params.vk_g1, params.vk_g2, params.ic)
+
+    @property
+    def n_public(self):
+        return self.ic.n - 1
+
+    def verify(self, proofs, inputs, rho=None):
+        """proofs: a list of (A, B, C) as `prove` / `prove_r1cs` return them ((9,), (17,), (9,) uint64; extra items such as q are ignored), or a
+        (k, 35) array.  inputs: (k, n_public, 4) Montgomery Fr, or per proof a list of Python ints — the instance without its leading one.
+        rho: (k, 2) uint64 128-bit non-zero batching weights; None draws them from os.urandom (zeros redrawn).  -> (k,) bool"""
+        if isinstance(proofs, np.ndarray):
+            arr = np.ascontiguousarray(proofs, dtype=np.uint64).reshape(-1, 35)
+        else:
+            arr = np.stack([np.concatenate([np.asarray(p[0], dtype=np.uint64).reshape(9), np.asarray(p[1], dtype=np.uint64).reshape(17),
+                                            np.asarray(p[2], dtype=np.uint64).reshape(9)]) for p in proofs]) if len(proofs) else np.zeros((0, 35), np.uint64)
+        k = arr.shape[0]
+        if isinstance(inputs, np.ndarray):
+            xs = np.ascontiguousarray(inputs, dtype=np.uint64).reshape(k, self.n_public, 4)
+        else:
+            rows = [list(r) for r in inputs]
+            if len(rows) != k or any(len(r) != self.n_public for r in rows):
+                raise ValueError(f"inputs: {k} rows of {self.n_public} public inputs expected")
+            xs = np.stack([_mont([int(v) for v in r]) for r in rows]) if k and self.n_public else np.zeros((k, self.n_public, 4), np.uint64)
+        if rho is None and k >= 2:
+            rho = np.zeros((k, 2), dtype=np.uint64)
+            for i in range(k):
+                while not rho[i].any():
+                    rho[i] = np.frombuffer(os.urandom(16), dtype=np.uint64)
+        return groth16_verify(self.vk_g1, self.vk_g2, self.ic, arr, xs, rho if k >= 2 else None)
+
+    def free(self):
+        if self._own_ic:
+            self.ic.free()

@@ -206,6 +206,50 @@ def groth16_setup_timing():
     return dict(zip(keys, [float(x) for x in ms]))
 
 
+def _pair_rows(g1, g2):
+    g1 = _c(g1).reshape(-1, 9)
+    g2 = _c(g2).reshape(-1, 17)
+    if g1.shape[0] != g2.shape[0]:
+        raise ValueError("g1 and g2 must hold the same number of points")
+    return g1, g2
+
+
+def pairing(g1, g2):
+    """kgr_pairing op 0: the reduced optimal-ate pairing e(P_i, Q_i) per pair.  g1: (n, 9) x, y, is_infinity; g2: (n, 17) x.c0 x.c1 y.c0 y.c1,
+    is_infinity (Montgomery).  -> (n, 48) uint64: 12 Montgomery Fq elements per value in tower order (include/kgr_msm.h)."""
+    _lib.ensure_init()
+    g1, g2 = _pair_rows(g1, g2)
+    out = np.zeros((g1.shape[0], 48), dtype=np.uint64)
+    _lib.check(_lib.lib().kgr_pairing(_u64(g1), _u64(g2), g1.shape[0], 0, _u64(out)))
+    return out
+
+
+def pairing_product(g1, g2):
+    """kgr_pairing op 1: prod_i e(P_i, Q_i) with one final exponentiation.  -> (48,) uint64."""
+    _lib.ensure_init()
+    g1, g2 = _pair_rows(g1, g2)
+    out = np.zeros(48, dtype=np.uint64)
+    _lib.check(_lib.lib().kgr_pairing(_u64(g1), _u64(g2), g1.shape[0], 1, _u64(out)))
+    return out
+
+
+def groth16_verify(vk_g1, vk_g2, ic, proofs, inputs, rho):
+    """kgr_groth16_verify.  vk_g1 (3, 9), vk_g2 (3, 17), ic: Bases of n_public + 1 G1 points, proofs (k, 35), inputs (k, n_public, 4) Montgomery
+    Fr, rho (k, 2) uint64 or None.  -> (k,) bool."""
+    _lib.ensure_init()
+    vk_g1, vk_g2, proofs = _c(vk_g1).reshape(3, 9), _c(vk_g2).reshape(3, 17), _c(proofs).reshape(-1, 35)
+    k, n_public = proofs.shape[0], ic.n - 1
+    inputs = _c(inputs).reshape(k, n_public, 4) if n_public else np.zeros((k, 0, 4), dtype=np.uint64)
+    ok = np.zeros(k, dtype=np.uint32)
+    rp = None
+    if rho is not None:
+        rho = _c(rho).reshape(k, 2)
+        rp = _u64(rho)
+    _lib.check(_lib.lib().kgr_groth16_verify(_u64(vk_g1), _u64(vk_g2), ic._h, _u64(proofs), k, _u64(inputs) if inputs.size else None, n_public, rp,
+                                             ok.ctypes.data_as(ctypes.POINTER(ctypes.c_uint32))))
+    return ok.astype(bool)
+
+
 def msm_device(bases, d_scalars_ptr, n, scalar_fmt=SCALARS_MONTGOMERY, base_off=0):
     """MSM with the scalars already in device memory (raw pointer, n x 4 uint64)."""
     out = np.zeros(3 * coord_limbs(bases.curve), dtype=np.uint64)

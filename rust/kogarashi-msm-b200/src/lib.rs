@@ -86,6 +86,9 @@ extern "C" {
                          l: *mut *mut kgr_bases_t, a: *mut *mut kgr_bases_t, b_g1: *mut *mut kgr_bases_t, b_g2: *mut *mut kgr_bases_t,
                          ic: *mut *mut kgr_bases_t, vk_g1: *mut u64, vk_g2: *mut u64) -> i32;
     fn kgr_groth16_setup_last_timing(ms: *mut f32) -> i32;
+    fn kgr_pairing(g1: *const u64, g2: *const u64, n: usize, op: i32, out: *mut u64) -> i32;
+    fn kgr_groth16_verify(vk_g1: *const u64, vk_g2: *const u64, ic: *mut kgr_bases_t, proofs: *const u64, k: usize, inputs: *const u64,
+                          n_public: usize, rho: *const u64, ok: *mut u32) -> i32;
     fn kgr_set_param(name: *const c_char, value: c_long) -> i32;
     fn kgr_last_timing(dev: i32, ms: *mut f32, shape: *mut u32) -> i32;
     fn kgr_event_record(dev: i32, idx: i32) -> i32;
@@ -572,5 +575,36 @@ mod unused {
                  kgr_set_param as usize, kgr_last_timing as usize, kgr_event_record as usize, kgr_event_elapsed_ms as usize, kgr_launch_count as usize,
                  kgr_test_field_op as usize, kgr_test_point_op as usize, kgr_fixed_base_mul as usize, kgr_bases_generate as usize,
                  kgr_bases_generate_at as usize, kgr_microbench as usize);
+    }
+}
+
+/// `groth16/src/verifier.rs` on the GPU (`kgr_groth16_verify`, uncompiled like the rest of this file): the verifying key as the limbs `GpuParams`
+/// holds and the ic query borrowed from it.  `proofs`: per proof A[9] B[17] C[9] (x, y, is_infinity; Montgomery limbs); `inputs`: per proof the
+/// public inputs without the leading one.  For two or more proofs one batched pairing check runs with the caller's 128-bit weights `rho`
+/// (non-zero, unpredictable to the prover); if it fails, every proof is checked on its own.
+pub struct GpuVerifier<'a> {
+    pub vk_g1: [u64; 27],
+    pub vk_g2: [u64; 51],
+    pub ic: &'a RegisteredBases<bn_254::G1Affine>,
+}
+
+impl<'a> GpuVerifier<'a> {
+    pub fn from_params(params: &'a GpuParams) -> Self {
+        Self { vk_g1: params.vk_g1, vk_g2: params.vk_g2, ic: &params.ic }
+    }
+
+    pub fn verify(&self, proofs: &[[u64; 35]], inputs: &[Vec<bn_254::Fr>], rho: &[[u64; 2]]) -> Vec<bool> {
+        let k = proofs.len();
+        let n_public = self.ic.len - 1;
+        assert!(inputs.len() == k && inputs.iter().all(|x| x.len() == n_public));
+        let flat_p: Vec<u64> = proofs.iter().flat_map(|p| p.iter().copied()).collect();
+        let flat_x: Vec<u64> = inputs.iter().flat_map(|x| x.iter().flat_map(|s| s.0)).collect();
+        let flat_r: Vec<u64> = rho.iter().flat_map(|r| r.iter().copied()).collect();
+        let mut ok = vec![0u32; k];
+        check(unsafe {
+            kgr_groth16_verify(self.vk_g1.as_ptr(), self.vk_g2.as_ptr(), self.ic.handle, flat_p.as_ptr(), k, flat_x.as_ptr(), n_public,
+                               if k >= 2 { flat_r.as_ptr() } else { core::ptr::null() }, ok.as_mut_ptr())
+        });
+        ok.into_iter().map(|v| v != 0).collect()
     }
 }
