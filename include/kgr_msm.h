@@ -174,6 +174,23 @@ int kgr_pedersen_commit_vec(kgr_bases_t *ck, const kgr_vec_t *m, size_t sc_off, 
 /* kgr_nova_cross_term with z1, z2 resident (n_z elements each) and T left in the resident vector t (m elements; NULL: internal buffer).
  * With ck != NULL also commit(T).  No host <-> device traffic except the 72-byte commitment. */
 int kgr_nova_cross_term_device(kgr_r1cs_t *shape, const kgr_vec_t *z1, const kgr_vec_t *z2, kgr_vec_t *t, kgr_bases_t *ck, uint64_t *commit_out);
+/* R1csShape::is_sat (strict, e == NULL) / the relaxed check (e != NULL) on resident vectors (nova/src/relaxed_r1cs.rs:80-146): for every row
+ * i < m, (A z)_i (B z)_i = u (C z)_i + E_i with z = (u, x, w) flat (z->n >= n_z), u = z[0] and E = e[0, m) when relaxed, u = 1 and E = 0 when
+ * strict.  W = z[w_off, n_z).  With ck (a BN254 G1 or Grumpkin key whose scalar field is the shape's field, one shard on the first device):
+ * commit(W) is compared with commit_w and commit(E) with commit_e, each zipped with ck.g (pedersen.rs:15-20, min length) and compared as zkstd
+ * compares affine points (group.rs:5-13: an identity equals only an identity, otherwise x and y limb for limb).  Expected commitments use the
+ * layout kgr_pedersen_commit* returns, x[4] y[4] is_infinity.  Either may be NULL, which skips that check: which commitments the reference's
+ * relaxed check re-derives (W only, or W and E) is not recorded here, so the caller chooses; the strict check re-derives commit(W) (:143).
+ * The relation runs on the library's stream, the two MSMs on two further lanes at the same time ("lane_threads" as kgr_groth16_msms).  Work
+ * enqueued on the library's stream before the call (a fold or cross term writing z or e) is complete before z or e is read.
+ * report[6]: [0] sat (1 iff every check made holds)  [1] rows violating (A z)o(B z) = u (C z) + E  [2] first violating row (m if none)
+ *            [3] commit(W) == commit_w: 1 equal, 0 different, 2 not checked  [4] commit(E) == commit_e: same  [5] u: 1 if relaxed or z[0] == 1
+ * An unsatisfied instance is KGR_OK with report[0] == 0, not an error.
+ * Refused with KGR_E_ARG before any work: a NULL shape, z or report; a shape, vector or key from before the last kgr_init; vector fields that
+ * differ from the shape's; a ck of another scalar field, another curve or more than one shard; z->n < n_z or e->n < m; w_off outside 1 .. n_z;
+ * commit_w or commit_e without ck; commit_e in strict mode. */
+int kgr_nova_is_sat(const kgr_r1cs_t *shape, const kgr_vec_t *z, const kgr_vec_t *e, size_t w_off, kgr_bases_t *ck,
+                    const uint64_t *commit_w /* [9] or NULL */, const uint64_t *commit_e /* [9] or NULL */, uint64_t *report /* [6] */);
 
 /* Page-locked host memory for callers that marshal into a reusable arena instead of a fresh pageable buffer per call (a Rust Vec is
  * pageable: the library then stages it through its own pinned ring, one extra copy).  cudaHostAlloc / cudaFreeHost underneath. */

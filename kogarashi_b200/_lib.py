@@ -20,7 +20,7 @@ EXPORTS = [
     "kgr_event_elapsed_ms", "kgr_launch_count", "kgr_bases_precompute", "kgr_ntt", "kgr_ntt_device", "kgr_groth16_h",
     "kgr_bases_generate_at", "kgr_vec_upload", "kgr_vec_download", "kgr_vec_free", "kgr_vec_len", "kgr_vec_write", "kgr_vec_fold_device", "kgr_msm_vec",
     "kgr_pedersen_commit_vec", "kgr_nova_cross_term_device", "kgr_host_alloc", "kgr_host_free", "kgr_msm_batch", "kgr_groth16_msms", "kgr_groth16_prove_r1cs", "kgr_groth16_setup", "kgr_groth16_setup_last_timing", "kgr_r1cs_register", "kgr_r1cs_free", "kgr_r1cs_mul", "kgr_nova_cross_term", "kgr_r1cs_last_timing", "kgr_vec_fold",
-    "kgr_pairing", "kgr_groth16_verify",
+    "kgr_pairing", "kgr_groth16_verify", "kgr_nova_is_sat",
 ]
 
 
@@ -100,6 +100,7 @@ def lib():
     L.kgr_msm_vec.argtypes = [vp, sz, vp, sz, sz, u64p]
     L.kgr_pedersen_commit_vec.argtypes = [vp, vp, sz, sz, u64p]
     L.kgr_nova_cross_term_device.argtypes = [vp, vp, vp, vp, vp, u64p]
+    L.kgr_nova_is_sat.argtypes = [vp, vp, vp, sz, vp, u64p, u64p, u64p]
     L.kgr_host_alloc.argtypes = [sz, ctypes.POINTER(vp)]
     L.kgr_host_free.argtypes = [vp]
     L.kgr_pairing.argtypes = [u64p, u64p, sz, ci, u64p]

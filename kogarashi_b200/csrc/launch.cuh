@@ -106,6 +106,10 @@ struct LaunchR1cs {
     static void spmv(cudaStream_t st, int field, uint32_t m, const Csr &mat, const uint32_t *z, uint32_t *out);
     static void cross_term(cudaStream_t st, int field, uint32_t m, const Csr &a, const Csr &b, const Csr &c, const uint32_t *z1, const uint32_t *z2, uint32_t *t);
     static void vec_fold(cudaStream_t st, int field, uint32_t n, const uint32_t *a, const uint32_t *b, const uint32_t r8[8], uint32_t *out);
+    // (A z) o (B z) = u (C z) + E row by row (e == nullptr: E = 0; strict: u = 1).  result: 3 words, on entry {0, 0xFFFFFFFF, 0}; on exit
+    // [0] violating rows, [1] the first of them (0xFFFFFFFF if none), [2] strict only: z[0] == 1
+    static void relaxed_check(cudaStream_t st, int field, uint32_t m, const Csr &a, const Csr &b, const Csr &c, const uint32_t *z, const uint32_t *e,
+                              bool strict, uint32_t *result);
     // Groth16 (Fr only): A z, B z, C z over 2^k positions, zero padded, each stored at its bit-reversed index of out[0..2] (2^k elements each)
     static void evaluate(cudaStream_t st, uint32_t k, uint32_t m, const Csr &a, const Csr &b, const Csr &c, const uint32_t *z, uint32_t *const out[3]);
 };

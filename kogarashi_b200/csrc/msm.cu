@@ -192,6 +192,7 @@ struct Engine {
     uint64_t launches = 0;            // kernels of this library launched on this engine since init
     cudaEvent_t user_ev[4] = {};      // kgr_event_record / kgr_event_elapsed_ms
     cudaEvent_t aux_ev[3] = {};       // phase marks of the R1CS calls (kgr_r1cs_last_timing)
+    DevBuf<uint32_t> sat_result;      // kgr_nova_is_sat: violation count, first violating row, z[0] == 1
     DevBuf<uint8_t> oneshot_pts, oneshot_inf;  // device copy of the bases of kgr_msm_oneshot
     std::map<uint32_t, std::shared_ptr<struct NttDomain>> ntt_domains;  // per log2(n): twiddle / coset tables in HBM
     DevBuf<uint8_t> ntt_buf[3];
@@ -245,6 +246,7 @@ struct Engine {
         for (auto &x : ev_piece_pts) if (x) { cudaEventDestroy(x); x = nullptr; }
         for (auto &e : user_ev) if (e) cudaEventDestroy(e);
         for (auto &e : aux_ev) if (e) cudaEventDestroy(e);
+        sat_result.release();
         oneshot_pts.release(); oneshot_inf.release();
         ntt_domains.clear();
         for (auto &b : ntt_buf) b.release();
@@ -2474,6 +2476,114 @@ int kgr_groth16_prove_r1cs(unsigned log_n, const kgr_r1cs_t *cs, const kgr_vec_t
         for (auto &t : th) t.join();
         for (auto &ce : errs)
             if (ce.e != cudaSuccess) throw ce;
+        return KGR_OK;
+    });
+}
+
+// ---- Nova: R1csShape::is_sat / is_sat_relaxed on resident vectors (nova/src/relaxed_r1cs.rs:80-146) -----------------------------------------
+// zkstd affine equality (macros/curve/weierstrass/group.rs:5-13) of two x[4] y[4] is_infinity values: an identity equals only an identity
+static bool affine_eq9(const uint64_t *a, const uint64_t *b) {
+    if (a[8] || b[8]) return a[8] && b[8];
+    return std::memcmp(a, b, 64) == 0;
+}
+
+int kgr_nova_is_sat(const kgr_r1cs_t *s, const kgr_vec_t *z, const kgr_vec_t *e, size_t w_off, kgr_bases_t *ck, const uint64_t *commit_w,
+                    const uint64_t *commit_e, uint64_t *report) {
+    std::lock_guard<std::mutex> lk(g_mu);
+    if (g_engines.empty()) return fail(KGR_E_NOT_INIT, "kgr_init has not been called");
+    if (!s || !z || !report) return fail(KGR_E_ARG, "null pointer");
+    if (int rc = vec_check(z)) return rc;
+    if (e)
+        if (int rc = vec_check(e)) return rc;
+    if (s->generation != g_generation) return fail(KGR_E_ARG, "R1CS shape was registered before the last kgr_init");
+    if (z->field != s->field || (e && e->field != s->field)) return fail(KGR_E_ARG, "vector field does not match the R1CS field");
+    if (z->n < s->n_z || (e && e->n < s->m)) return fail(KGR_E_ARG, "vector shorter than the shape needs");
+    if (w_off < 1 || w_off > s->n_z) return fail(KGR_E_ARG, "w_off must be in 1 .. n_z (W = z[w_off ..] follows u and x)");
+    if ((commit_w || commit_e) && !ck) return fail(KGR_E_ARG, "an expected commitment needs the commitment key");
+    if (commit_e && !e) return fail(KGR_E_ARG, "commit_e in strict mode: there is no E");
+    if (ck) {
+        if (ck->curve != KGR_CURVE_BN254_G1 && ck->curve != KGR_CURVE_GRUMPKIN) return fail(KGR_E_ARG, "the commitment key must be a BN254 G1 or Grumpkin vector");
+        if ((ck->curve == KGR_CURVE_GRUMPKIN ? 0 : 1) != s->field) return fail(KGR_E_ARG, "commitment key curve does not match the R1CS field");
+        if (ck->generation != g_generation) return fail(KGR_E_ARG, "base handle was created before the last kgr_init");
+        if (ck->shards.size() != 1 || ck->shards[0].eng != 0) return fail(KGR_E_ARG, "the commitment key must live on the first device only");
+    }
+    const Params P = t_params;
+    return guarded([&]() -> int {
+        uint64_t rep[6] = {0, 0, 0, 2, 2, 1};
+        struct Commit {
+            const uint32_t *d_sc;  // the committed vector in device memory
+            size_t n;              // pairs: zip with ck.g (pedersen.rs:16-17)
+            const uint64_t *expect;
+            uint64_t *status;
+        };
+        std::vector<Commit> work;
+        if (commit_w) work.push_back(Commit{z->d.p + 8 * w_off, std::min(s->n_z - w_off, ck->n), commit_w, &rep[3]});
+        if (commit_e) work.push_back(Commit{e->d.p, std::min(s->m, ck->n), commit_e, &rep[4]});
+        ensure_lanes(0, 1 + work.size());
+        Engine &e0 = g_engines[0];
+        CK(cudaSetDevice(e0.dev));
+        CK(cudaEventRecord(e0.ev_input, e0.st));  // z and E are complete once this event is: the commitment lanes wait for it before reading them
+        // lane 0: the relation.  It runs no MSM in this call, so its pinned result buffer takes the three result words.
+        uint32_t *res = e0.h_result;
+        auto relation_start = [&]() {
+            e0.sat_result.ensure(3);
+            CK(cudaMemsetAsync(e0.sat_result.p, 0, 3 * sizeof(uint32_t), e0.st));
+            CK(cudaMemsetAsync(e0.sat_result.p + 1, 0xFF, sizeof(uint32_t), e0.st));
+            LaunchR1cs::relaxed_check(e0.st, s->field, (uint32_t)s->m, s->csr(0), s->csr(1), s->csr(2), z->d.p, e ? e->d.p : nullptr, !e, e0.sat_result.p);
+            e0.launches++;
+            CK(cudaGetLastError());
+            CK(cudaMemcpyAsync(res, e0.sat_result.p, 3 * sizeof(uint32_t), cudaMemcpyDeviceToHost, e0.st));
+        };
+        auto relation_finish = [&]() {
+            CK(cudaSetDevice(e0.dev));
+            CK(cudaStreamSynchronize(e0.st));
+        };
+        // lanes 1, 2: commit(W), commit(E) from the resident scalars
+        auto commit_start = [&](const Commit &c, Engine &ln) {
+            if (c.n) with_curve(ck->curve, [&](auto tag) { lane_start_device<std::remove_pointer_t<decltype(tag)>>(ln, P, ck->shards[0], 0, c.d_sc, c.n, e0.ev_input); });
+        };
+        auto commit_finish = [&](const Commit &c, Engine &ln) {
+            uint64_t proj[24], aff[17];
+            with_curve(ck->curve, [&](auto tag) {
+                typedef std::remove_pointer_t<decltype(tag)> C;
+                if (c.n) lane_finish<C>(ln, proj);
+                else combine_partials<C>(std::vector<Partial>(), proj);
+                proj_to_affine_host<C>(proj, aff);
+            });
+            *c.status = affine_eq9(aff, c.expect) ? 1 : 0;
+        };
+        if (!P.lane_threads) {
+            relation_start();
+            for (size_t j = 0; j < work.size(); j++) commit_start(work[j], lane_of(0, 1 + j));
+            relation_finish();
+            for (size_t j = 0; j < work.size(); j++) commit_finish(work[j], lane_of(0, 1 + j));
+        } else {
+            std::vector<CudaError> errs(1 + work.size(), CudaError{cudaSuccess, "", 0});
+            std::vector<std::thread> th;
+            for (size_t j = 0; j < work.size(); j++)
+                th.emplace_back([&, j]() {
+                    try {
+                        commit_start(work[j], lane_of(0, 1 + j));
+                        commit_finish(work[j], lane_of(0, 1 + j));
+                    } catch (CudaError &ce) {
+                        errs[1 + j] = ce;
+                    }
+                });
+            try {
+                relation_start();
+                relation_finish();
+            } catch (CudaError &ce) {
+                errs[0] = ce;
+            }
+            for (auto &t : th) t.join();
+            for (auto &ce : errs)
+                if (ce.e != cudaSuccess) throw ce;
+        }
+        rep[1] = res[0];
+        rep[2] = res[0] ? res[1] : s->m;
+        if (!e) rep[5] = res[2];
+        rep[0] = (rep[1] == 0 && rep[5] == 1 && rep[3] != 0 && rep[4] != 0) ? 1 : 0;
+        std::memcpy(report, rep, sizeof rep);
         return KGR_OK;
     });
 }

@@ -63,6 +63,21 @@ template <class P> KGR_HD void body_cross_term(uint32_t i, uint32_t m, const Csr
     el_store(t + 8 * (size_t)i, r);
 }
 
+// R1csShape::is_sat_relaxed / is_sat, one row (nova/src/relaxed_r1cs.rs:80-146): true iff row i VIOLATES (A z)_i (B z)_i = u (C z)_i + E_i.
+// u = z[0], or the constant one when strict (is_sat); e == nullptr: E = 0.  Rows i >= m never violate.
+template <class P>
+KGR_HD bool body_relaxed_row(uint32_t i, uint32_t m, const Csr &a, const Csr &b, const Csr &c, const uint32_t *z, const uint32_t *e, bool strict) {
+    if (i >= m) return false;
+    const uint32_t *zs[1] = {z};
+    Fp<P> az, bz, cz;
+    row_dot<P, 1>(a, i, zs, &az);
+    row_dot<P, 1>(b, i, zs, &bz);
+    row_dot<P, 1>(c, i, zs, &cz);
+    Fp<P> rhs = strict ? cz : fp_mul(ld_elem<P>(z, 0), cz);
+    if (e) rhs = fp_add(rhs, ld_elem<P>(e, i));
+    return !fp_eq(fp_mul(az, bz), rhs);
+}
+
 // The k low bits of i reversed (fft.rs:157-162 swaps i and this index)
 KGR_HD uint32_t bitrev_k(uint32_t i, uint32_t k) {
 #ifdef __CUDA_ARCH__

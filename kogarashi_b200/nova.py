@@ -5,9 +5,11 @@ Reference:
   nova/src/prover.rs:53-90                  Prover::compute_cross_term          T = AZ1∘BZ2 + AZ2∘BZ1 − u1·CZ2 − u2·CZ1
   nova/src/prover.rs:35                     self.ck.commit(&t)
   nova/src/relaxed_r1cs/witness.rs:56-71    RelaxedR1csWitness::fold            e = e1 + t·r,  w = w1 + w2·r
+  nova/src/relaxed_r1cs.rs:80-146           R1csShape::is_sat(_relaxed)         (A z)∘(B z) = u·(C z) + E, commit(W) (and commit(E))
 Vectors are (n, 4) uint64 Montgomery arrays of the constraint system's field (FIELD_FQ for nova's GrumpkinDriver, FIELD_FR
 for Bn254Driver); z = (u, x, w) is passed whole, matrices are CSR over flat column indices into z.
 """
+import collections
 import ctypes
 
 import numpy as np
@@ -18,6 +20,20 @@ from .msm import _c, _u64
 FIELD_FQ, FIELD_FR = 0, 1
 _u32p = ctypes.POINTER(ctypes.c_uint32)
 _u64p = ctypes.POINTER(ctypes.c_uint64)
+
+
+class SatReport(collections.namedtuple("SatReport", "sat violations first_violation commit_w commit_e u_ok")):
+    """kgr_nova_is_sat's report.  `bool(report)` is `sat`.  violations: rows with (A z)_i (B z)_i != u (C z)_i + E_i; first_violation: the
+    lowest such row (m if none); commit_w / commit_e: True equal, False different, None not checked; u_ok: relaxed, or z[0] == 1."""
+    __slots__ = ()
+
+    def __bool__(self):
+        return self.sat
+
+    @classmethod
+    def _from_words(cls, r):
+        status = {0: False, 1: True, 2: None}
+        return cls(bool(r[0]), int(r[1]), int(r[2]), status[int(r[3])], status[int(r[4])], bool(r[5]))
 
 
 class R1csShape:
@@ -60,6 +76,24 @@ class R1csShape:
         _lib.check(_lib.lib().kgr_nova_cross_term(self._h, _u64(z1), _u64(z2), _u64(t) if t is not None else None,
                                                   bases._h if bases is not None else None, _u64(commit) if commit is not None else None))
         return (t, commit) if bases is not None else t
+
+    def is_sat(self, z, w_off, ck=None, commit_w=None):
+        """R1csShape::is_sat (relaxed_r1cs.rs:117-146) on the resident z = (1, x, w) (`DeviceVec`): (A z) o (B z) = C z for every row, and
+        with a key (`Bases` or `PedersenCommitment`) commit(z[w_off ..]) == commit_w when commit_w (9,) is given.  -> SatReport"""
+        return self._is_sat(z, None, w_off, ck, commit_w, None)
+
+    def is_sat_relaxed(self, z, e, w_off, ck=None, commit_w=None, commit_e=None):
+        """The relaxed relation (relaxed_r1cs.rs:80-114): (A z) o (B z) = u (C z) + E with u = z[0], z and E resident (`DeviceVec`); each
+        expected commitment is checked only when given.  -> SatReport"""
+        return self._is_sat(z, e, w_off, ck, commit_w, commit_e)
+
+    def _is_sat(self, z, e, w_off, ck, commit_w, commit_e):
+        bases = getattr(ck, "g", ck)
+        keep = [_c(c).reshape(9) if c is not None else None for c in (commit_w, commit_e)]
+        report = np.zeros(6, dtype=np.uint64)
+        _lib.check(_lib.lib().kgr_nova_is_sat(self._h, z._h, e._h if e is not None else None, w_off, bases._h if bases is not None else None,
+                                              *[_u64(c) if c is not None else None for c in keep], _u64(report)))
+        return SatReport._from_words(report)
 
     def last_timing(self):
         ms = (ctypes.c_float * 3)()

@@ -75,6 +75,8 @@ extern "C" {
     fn kgr_pedersen_commit_vec(ck: *mut kgr_bases_t, m: *const kgr_vec_t, sc_off: usize, n: usize, out: *mut u64) -> i32;
     fn kgr_nova_cross_term_device(shape: *mut kgr_r1cs_t, z1: *const kgr_vec_t, z2: *const kgr_vec_t, t: *mut kgr_vec_t, ck: *mut kgr_bases_t,
                                   commit_out: *mut u64) -> i32;
+    fn kgr_nova_is_sat(shape: *const kgr_r1cs_t, z: *const kgr_vec_t, e: *const kgr_vec_t, w_off: usize, ck: *mut kgr_bases_t, commit_w: *const u64,
+                       commit_e: *const u64, report: *mut u64) -> i32;
     fn kgr_host_alloc(bytes: usize, out: *mut *mut c_void) -> i32;
     fn kgr_host_free(p: *mut c_void) -> i32;
     fn kgr_groth16_msms(log_n: u32, a: *const u64, b: *const u64, c: *const u64, m: usize, h: *mut kgr_bases_t, h_out: *mut u64, q_out: *mut u64,
@@ -541,6 +543,25 @@ impl R1csShapeGpu {
         let mut t = vec![0u64; 4 * self.m];
         check(unsafe { kgr_nova_cross_term(self.handle, z1.as_ptr(), z2.as_ptr(), t.as_mut_ptr(), core::ptr::null_mut(), core::ptr::null_mut()) });
         t
+    }
+    /// `R1csShape::is_sat` (nova/src/relaxed_r1cs.rs:117-146) on the resident z = (1, x, w): (A z) o (B z) = C z row by row and, with a key,
+    /// commit(z[w_off ..]) == commit_w.  `report` as `kgr_nova_is_sat`: [0] sat, [1] violating rows, [2] first of them (m if none), [3] commit(W)
+    /// 1 equal / 0 different / 2 not checked, [4] 2, [5] z[0] == 1.
+    pub fn is_sat<C: GpuCurve>(&self, z: &DeviceVec, w_off: usize, ck: Option<(&RegisteredBases<C>, &[u64; 9])>) -> [u64; 6] {
+        let mut report = [0u64; 6];
+        let (key, cw) = ck.map_or((core::ptr::null_mut(), core::ptr::null()), |(b, c)| (b.handle, c.as_ptr()));
+        check(unsafe { kgr_nova_is_sat(self.handle, z.handle, core::ptr::null(), w_off, key, cw, core::ptr::null(), report.as_mut_ptr()) });
+        report
+    }
+    /// The relaxed relation (relaxed_r1cs.rs:80-114), u = z[0], with E resident; each expected commitment is optional (`None` skips that check).
+    pub fn is_sat_relaxed<C: GpuCurve>(&self, z: &DeviceVec, e: &DeviceVec, w_off: usize, ck: Option<&RegisteredBases<C>>, commit_w: Option<&[u64; 9]>,
+                                       commit_e: Option<&[u64; 9]>) -> [u64; 6] {
+        let mut report = [0u64; 6];
+        let key = ck.map_or(core::ptr::null_mut(), |b| b.handle);
+        let cw = commit_w.map_or(core::ptr::null(), |c| c.as_ptr());
+        let ce = commit_e.map_or(core::ptr::null(), |c| c.as_ptr());
+        check(unsafe { kgr_nova_is_sat(self.handle, z.handle, e.handle, w_off, key, cw, ce, report.as_mut_ptr()) });
+        report
     }
     /// SparseMatrix::prod (zkstd/src/matrix.rs:36-48): which = 0 A, 1 B, 2 C
     pub fn prod(&self, which: i32, z: &[u64]) -> Vec<u64> {
